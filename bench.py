@@ -12,6 +12,7 @@ dealt round-robin to the ranks, every rank pastes / histograms only the pixels i
 sums the per-image integer histograms before every rank scans them.
 
   python bench.py [--gpus N --steps K --warmup W]          B200 path (one rank per GPU under torchrun)
+  python bench.py [...] --dump-outputs DIR                 + the last timed image's maps (sample) and scores as .npy
   python bench.py --impl reference [...]                   the reference's CPU path (oracle port) on host cores
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is obtained.
@@ -183,7 +184,8 @@ def run_b200(args):
         """`count` images of the set (strong scaling: the same images for every N), (image, tile) units over
         the ranks in groups of `world` images.  host=False: inputs resident in HBM, results stay on the device
         (value).  host=True: each group's images + masks come from pinned host memory, the assembled
-        probability maps and the scores go back to pinned host memory (e2e)."""
+        probability maps and the scores go back to pinned host memory (e2e).
+        -> (scores per lesion model, {lesion: this rank's pieces of the probability map of image count-1})"""
         hist = torch.zeros((len(LESIONS), count, 2, _lib.PR_BINS), dtype=torch.int32, device=dev)
         strad = torch.zeros((len(LESIONS), count, _lib.PR_NTHRESH, 2), dtype=torch.int32, device=dev)
         main = torch.cuda.current_stream()
@@ -202,6 +204,7 @@ def run_b200(args):
             return group, imgs, gts, ev
 
         pending = upload(starts[0]) if host else None
+        last_maps = {}
         for gi, g in enumerate(starts):
             if host:
                 group, imgs, gts, ev = pending
@@ -216,6 +219,8 @@ def run_b200(args):
             for li, les in enumerate(LESIONS):
                 canvases, _ = drv.partitioned_group(models[les], tfm, imgs, gts[les], S, mean, std, hist[li], strad[li],
                                                     g, rank, world, args.tiles, unit_offset=g * TILES)
+                if group[-1] == count - 1:
+                    last_maps[les] = canvases[-1]
                 if host:
                     for r, i in enumerate(group):
                         if world > 1:
@@ -244,7 +249,7 @@ def run_b200(args):
         if world > 1:
             torch.cuda.current_stream().synchronize()
             allreduce_ms.append(a0.elapsed_time(a1))
-        return out
+        return out, last_maps
 
     def barrier():
         if world > 1:
@@ -276,12 +281,13 @@ def run_b200(args):
             dist.reduce(torch.zeros((4, 4), device=dev), dst=0)
 
     def timed(host):
-        run_set(args.warmup, host)                 # W warm-up steps (images)
+        if args.warmup:
+            run_set(args.warmup, host)             # W warm-up steps (images)
         barrier()
         before = K.LAUNCHES[0]
         t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         t0.record()
-        out = run_set(args.steps, host)            # EXACTLY `steps` images
+        out, maps = run_set(args.steps, host)      # EXACTLY `steps` images
         t1.record()
         barrier()
         launches = K.LAUNCHES[0] - before
@@ -290,8 +296,8 @@ def run_b200(args):
             mx = ms.clone()
             dist.all_reduce(mx, op=dist.ReduceOp.MAX)
             dist.all_reduce(ms, op=dist.ReduceOp.SUM)
-            return float(mx[0]), int(ms[1]), out
-        return float(ms[0]), int(ms[1]), out
+            return float(mx[0]), int(ms[1]), out, maps
+        return float(ms[0]), int(ms[1]), out, maps
 
     # the two HBM-bound kernels are timed ALONE, before the long tensor-bound run puts the GPU under its power cap
     # (their denominator is the burst copy bandwidth of MEASURED_PEAKS.json, also measured on an otherwise idle GPU)
@@ -310,10 +316,12 @@ def run_b200(args):
         blend_roof = blend_roofline(dev, hbm_peak, peak_src)
     prewarm()
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_total, launches, out = timed(False)
+    ms_total, launches, out, maps = timed(False)
     clocks = sampler.stop() if sampler else None
     ar_ms = allreduce_ms[-1] if allreduce_ms else 0.0
-    ms_e2e, _, _ = timed(True)
+    ms_e2e, _, _, _ = timed(True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, maps, rank, world)
 
     line = None
     if rank == 0:
@@ -355,6 +363,42 @@ def run_b200(args):
         dist.barrier()
         dist.destroy_process_group()
     return line
+
+
+DUMP_SAMPLE = 1 << 20                            # pixels per probability map in --dump-outputs (4 MB each)
+
+
+def dump_outputs(directory, out, maps, rank, world):
+    """--dump-outputs: what the resident timed run returned for its last image (step `steps`), per lesion model:
+    the same fixed sample of DUMP_SAMPLE pixels (numpy default_rng(0), row-major order) of the full-resolution
+    probability map as <lesion>_prob_sample.npy (float32), and the image's scores as float64: <lesion>_ap.npy,
+    <lesion>_roc.npy, <lesion>_threshold_counts.npy ([19, 2]: tp, pp per threshold), <lesion>_totals.npy
+    (n_pos, n_neg).  Under torchrun every rank holds only the pixels its tiles own: the pieces are summed onto
+    rank 0, which writes.  Two runs of one build are not bit-identical: the SE / SCSE channel means are summed with
+    float atomics in varying order (measured on a B200 at 1000 W, --steps 3 --warmup 2: up to 1.9e-3 in a
+    probability, 23 pixels in a threshold count, 1.2e-6 in an AP)."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    idx = np.sort(np.random.default_rng(0).choice(H * W, DUMP_SAMPLE, replace=False))
+    arrays = {}
+    for li, les in enumerate(LESIONS):
+        canvas = maps[les]
+        if world > 1:
+            dist.reduce(canvas, dst=0, op=dist.ReduceOp.SUM)
+        if rank != 0:
+            continue
+        flat = canvas[:, :W].reshape(-1)           # canvas rows are padded to a multiple of 4 columns
+        ap, roc, counts, totals = (t[-1] for t in out[li])
+        arrays[f"{les}_prob_sample"] = flat[torch.from_numpy(idx).to(flat.device)].float().cpu().numpy()
+        arrays[f"{les}_ap"] = ap.cpu().numpy()
+        arrays[f"{les}_roc"] = roc.cpu().numpy()
+        arrays[f"{les}_threshold_counts"] = counts.to(torch.float64).cpu().numpy()
+        arrays[f"{les}_totals"] = totals.to(torch.float64).cpu().numpy()
+    if rank == 0:
+        os.makedirs(directory, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def conv_roofline(model, tfm, image, mean, std, tiles, peak, peak_src):
@@ -691,10 +735,10 @@ def cpu_baseline():
 
 
 def run_reference(args):
-    """--impl reference: the reference's own CPU implementation of the path (here the oracle port; /root/reference
-    does not exist on the GPU box) on all host threads.  Each step RUNS one whole tile (8 D4 views, TTA mean,
-    sigmoid) and one full-image scoring; an image is 24 such tiles + 4 such scorings (stated in `config`).  Warm-up
-    = `warmup` single forwards.  Steps stop early after ~150 s of samples (the count actually run is reported)."""
+    """--impl reference: the reference's own CPU implementation of the path (here the oracle port) on all host
+    threads.  Each of the `steps` steps RUNS one whole tile (8 D4 views, TTA mean, sigmoid) and one full-image
+    scoring; an image is 24 such tiles + 4 such scorings (stated in `config`).  Warm-up = `warmup` single
+    forwards."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -702,12 +746,9 @@ def run_reference(args):
     for _ in range(args.warmup):
         cpu_tile_sample(threads, views=1, size=args.ref_size)
     tiles, scores = [], []
-    t_start = time.perf_counter()
-    for _ in range(max(1, args.steps)):
+    for _ in range(args.steps):
         tiles.append(cpu_tile_sample(threads, views=args.ref_views, size=args.ref_size) * (VIEWS / args.ref_views))
         scores.append(cpu_score_sample())
-        if time.perf_counter() - t_start > 150:
-            break
     t_tile, t_score = sum(tiles) / len(tiles), sum(scores) / len(scores)
     sec = TILES * len(LESIONS) * t_tile + len(LESIONS) * t_score
     value = 1.0 / sec
@@ -740,7 +781,11 @@ def main():
                          "quick contract tests, the printed value is then not a measurement)")
     ap.add_argument("--ref-views", type=int, default=VIEWS, choices=[1, VIEWS],
                     help="--impl reference: TTA views per sampled tile (8 = the workload; 1 only for quick contract tests)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the probability maps (fixed sample) and scores of the last timed image to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -232,3 +232,35 @@ def test_tta_patches_bf16_auc_within_1e3_of_reference_path(tmp_path, monkeypatch
     assert 0.05 < want_pr < 0.995, "degenerate test set"
     assert abs(seen["pr"] - want_pr) < 1e-3, (seen["pr"], want_pr)
     assert abs(seen["roc"] - want_roc) < 1e-3, (seen["roc"], want_roc)
+
+
+def test_bench_dump_outputs_hold_the_last_timed_image(tmp_path):
+    """cfg-4 (the bench workload) with ``--dump-outputs``: one JSON line on stdout, and DIR holds float32 / float64
+    arrays, 64 MB at most -- per lesion model a probability sample in [0, 1] and the scores of the last timed image;
+    with one timed image the dumped AP is the line's mean AP.  ``--warmup 0`` runs no warm-up set."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dump = tmp_path / "dump"
+    res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "1", "--warmup", "0",
+                          "--no-extra", "--no-cpu-baseline", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=1800)
+    assert res.returncode == 0, res.stderr[-3000:]
+    lines = [ln for ln in res.stdout.splitlines() if ln.strip()]
+    assert len(lines) == 1, res.stdout
+    line = json.loads(lines[0])
+    assert line["steps"] == 1 and line["warmup"] == 0
+    lesions = ("EX", "HE", "MA", "SE")
+    fields = ("prob_sample", "ap", "roc", "threshold_counts", "totals")
+    assert sorted(os.listdir(dump)) == sorted(f"{les}_{f}.npy" for les in lesions for f in fields)
+    assert sum(p.stat().st_size for p in dump.iterdir()) <= 64 << 20
+    for i, les in enumerate(lesions):
+        prob = np.load(dump / f"{les}_prob_sample.npy")
+        assert prob.dtype == np.float32 and prob.shape == (1 << 20,)
+        assert np.isfinite(prob).all() and prob.min() >= 0 and prob.max() <= 1 and prob.std() > 0
+        got = {f: np.load(dump / f"{les}_{f}.npy") for f in fields[1:]}
+        assert all(a.dtype == np.float64 for a in got.values())
+        assert got["threshold_counts"].shape == (19, 2) and got["totals"].sum() == 2848 * 4288
+        assert float(got["ap"]) == pytest.approx(line["config"]["mean_ap_per_lesion"][i], abs=1e-12)
