@@ -56,12 +56,15 @@ PROTOTYPES = {
     "eds_stem_conv7x7s2_mma": [_vp, _i, _i, _i, _i, C.POINTER(_i), _vp, _vp, _vp, _vp],
     "eds_conv2d_igemm_bf16": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],
     "eds_conv2d_igemm_bf16_gated": [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],
+    "eds_conv2d_igemm_grouped_supported": [_i, _i, _i, _i, _i, _i],
+    "eds_conv2d_igemm_bf16_grouped": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp],
     "eds_affine_rows": [_vp, _i, _i, _vp, _vp, _i, _vp, _vp],
     "eds_conv3x3_halo_supported": [_i, _i, _i, _i, _i, _i],
     "eds_conv3x3_halo_bf16": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp],
     "eds_conv3x3_small_supported": [_i, _i],
     "eds_conv3x3_small_bf16": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
     "eds_conv2d_simt": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp],
+    "eds_conv2d_simt_grouped": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp],
     "eds_head_conv3x3": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp],
     "eds_maxpool2d": [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _i, _vp],
     "eds_avgpool2_affine": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp],

@@ -9,7 +9,10 @@ Graphs restated (reference file:line under src/main/archs):
   proposed UNet++*   unetplusplusstar.py:341-352 (encoder), :239-263 (dense decoder),
                      :127-161 (decoder block), axial_attention_v2.py:261-281 (MHSA block)
   baseline UNet++    deep_supunetplusplus.py:116-139, :48-56  (+ smp encoders, 3P)
-  smp.Unet           3P (resnet34 encoder, 5 decoder blocks)
+  smp.Unet           3P (5 decoder blocks)
+  encoders (3P)      resnet34 (BasicBlock), resnet50 / resnext50_32x4d (torchvision Bottleneck, stride on the 3x3
+                     conv2), se_resnet50 (SEResNetBottleneck, stride on conv1), se_resnext50_32x4d
+                     (SEResNeXtBottleneck, stride on conv2); the 32-group 3x3 convolutions run on the grouped kernels
 """
 from __future__ import annotations
 
@@ -65,6 +68,7 @@ class Engine:
         self.act_dtype = torch.bfloat16 if precision == "bf16" else torch.float32
         self.conv_impl = "tc" if precision == "bf16" else "simt"
         self.w: Dict[str, object] = {}
+        self.groups: Dict[str, int] = {}        # grouped convolutions (ResNeXt conv2) -> groups
         self.features: Optional[Dict[str, torch.Tensor]] = None  # filled when keep_features is set
         self.keep_features = False
         # BatchNorm folding and repacking run on the HOST (IEEE fp32, same results as on the device): weight
@@ -78,7 +82,7 @@ class Engine:
             self.w["stem.packed"] = K.stem_pack_weights(self.w["stem"][0])
 
     # ------------------------------------------------------------ weight prep
-    def _conv(self, sd, name, conv_key, bn_key=None, perm=None):
+    def _conv(self, sd, name, conv_key, bn_key=None, perm=None, groups=1):
         w = sd[conv_key + ".weight"].float()
         if w.dim() == 3:
             w = w.unsqueeze(-1)
@@ -91,8 +95,12 @@ class Engine:
         if perm is not None:
             w = w[perm]
             b = None if b is None else b[perm]
-        self.w[name] = (w.permute(0, 2, 3, 1).contiguous().to(self.act_dtype),
-                        None if b is None else b.contiguous())
+        w = w.permute(0, 2, 3, 1).contiguous()
+        if groups > 1:
+            self.groups[name] = groups
+            if self.conv_impl == "tc":          # block-diagonal 64-channel operand, packed in fp32 before the cast
+                w = K.pack_grouped_weights(w)
+        self.w[name] = (w.to(self.act_dtype), None if b is None else b.contiguous())
 
     def _se(self, sd, name, fc1, fc2):
         w1, w2 = sd[fc1 + ".weight"].float(), sd[fc2 + ".weight"].float()
@@ -134,7 +142,7 @@ class Engine:
                 while f"encoder.layer{li}.{b}.conv1.weight" in sd:
                     p = f"encoder.layer{li}.{b}"
                     self._conv(sd, p + ".conv1", p + ".conv1", p + ".bn1")
-                    self._conv(sd, p + ".conv2", p + ".conv2", p + ".bn2")
+                    self._conv(sd, p + ".conv2", p + ".conv2", p + ".bn2", groups=self._conv2_groups(sd, p))
                     self._conv(sd, p + ".conv3", p + ".conv3", p + ".bn3")
                     # fp32 copy of the (rounded) conv3 weights as a [Cout][Cin] matrix: the SE squeeze from the
                     # channel means of conv3's input (K.affine_rows)
@@ -150,7 +158,9 @@ class Engine:
                 while f"encoder.layer{li}.{b}.conv1.weight" in sd:
                     p = f"encoder.layer{li}.{b}"
                     self._conv(sd, p + ".conv1", p + ".conv1", p + ".bn1")
-                    self._conv(sd, p + ".conv2", p + ".conv2", p + ".bn2")
+                    self._conv(sd, p + ".conv2", p + ".conv2", p + ".bn2", groups=self._conv2_groups(sd, p))
+                    if (p + ".conv3.weight") in sd:      # torchvision Bottleneck (resnet50, resnext50_32x4d)
+                        self._conv(sd, p + ".conv3", p + ".conv3", p + ".bn3")
                     if (p + ".downsample.0.weight") in sd:
                         self._conv(sd, p + ".downsample", p + ".downsample.0", p + ".downsample.1")
                     b += 1
@@ -172,7 +182,7 @@ class Engine:
             self.blocks = dense_decoder_blocks(enc_ch)
             bn_idx = 2
         else:
-            enc_ch = (3, 64, 256, 512, 1024, 2048) if self.senet else (3, 64, 64, 128, 256, 512)
+            enc_ch = self._encoder_channels(sd)
             if self.arch == "unetplusplus_deepsup":
                 self.blocks = dense_decoder_blocks(enc_ch)
             else:
@@ -203,9 +213,26 @@ class Engine:
         hw = sd["segmentation_head.0.weight"].float()
         self.w["head"] = (hw.permute(0, 2, 3, 1).contiguous(), sd["segmentation_head.0.bias"].float().contiguous())
 
+    @staticmethod
+    def _conv2_groups(sd, p):
+        """Groups of a block's 3x3 conv2 (input channels == output channels there): 32 for the ResNeXt blocks."""
+        w = sd[p + ".conv2.weight"]
+        return int(w.shape[0] // w.shape[1])
+
+    @staticmethod
+    def _encoder_channels(sd):
+        """(input, stem, layer1 .. layer4) channels of an smp encoder: the last conv of each stage's blocks."""
+        ch = [3, 64]
+        for li in range(1, 5):
+            p = f"encoder.layer{li}.0"
+            ch.append(int(sd[p + (".conv3.weight" if (p + ".conv3.weight") in sd else ".conv2.weight")].shape[0]))
+        return tuple(ch)
+
     # ---------------------------------------------------------------- kernels
     def _cv(self, x, name, stride=1, pad=0, relu=False, residual=None):
         w, b = self.w[name]
+        if name in self.groups:
+            return K.conv2d(x, w, b, stride, pad, relu, residual, impl=self.conv_impl, groups=self.groups[name])
         if isinstance(x, tuple):        # (upsampled part, skip part) of a decoder concat: two-input K loop
             return K.conv2d(x[0], w, b, stride, pad, relu, residual, impl=self.conv_impl, x1=x[1])
         return K.conv2d(x, w, b, stride, pad, relu, residual, impl=self.conv_impl)
@@ -306,8 +333,10 @@ class Engine:
 
     # ---------------------------------------------------------------- encoders
     def _se_bottleneck(self, p, x, stride):
-        out = self._cv(x, p + ".conv1", stride=stride, relu=True)
-        out = self._cv(out, p + ".conv2", pad=1, relu=True)
+        # SEResNetBottleneck strides its 1x1 conv1, SEResNeXtBottleneck (grouped conv2) its 3x3 conv2
+        s1, s2 = (1, stride) if (p + ".conv2") in self.groups else (stride, 1)
+        out = self._cv(x, p + ".conv1", stride=s1, relu=True)
+        out = self._cv(out, p + ".conv2", stride=s2, pad=1, relu=True)
         res = self._cv(x, p + ".downsample", stride=stride) if (p + ".downsample") in self.w else x
         if self.conv_impl == "tc" and SE_IN_EPILOGUE:
             # conv3 (1x1 + folded BN) has no activation, so the channel means its SE module squeezes are an affine
@@ -339,9 +368,15 @@ class Engine:
         while f"encoder.layer{li}.{b}.conv1" in self.w:
             p = f"encoder.layer{li}.{b}"
             s = stride if b == 0 else 1
-            out = self._cv(x, p + ".conv1", stride=s, pad=1, relu=True)
-            idt = self._cv(x, p + ".downsample", stride=s) if (p + ".downsample") in self.w else x
-            x = self._cv(out, p + ".conv2", pad=1, relu=True, residual=idt)
+            if (p + ".conv3") in self.w:        # torchvision Bottleneck: 1x1, 3x3 (stride, groups), 1x1 + identity
+                out = self._cv(x, p + ".conv1", relu=True)
+                out = self._cv(out, p + ".conv2", stride=s, pad=1, relu=True)
+                idt = self._cv(x, p + ".downsample", stride=s) if (p + ".downsample") in self.w else x
+                x = self._cv(out, p + ".conv3", relu=True, residual=idt)
+            else:                               # BasicBlock
+                out = self._cv(x, p + ".conv1", stride=s, pad=1, relu=True)
+                idt = self._cv(x, p + ".downsample", stride=s) if (p + ".downsample") in self.w else x
+                x = self._cv(out, p + ".conv2", pad=1, relu=True, residual=idt)
             b += 1
         return x
 

@@ -77,27 +77,47 @@ class ParamSpec:
 
 
 # ------------------------------------------------------------------- encoders
-def _se_bottleneck(s: ParamSpec, p, inplanes, planes, downsample):
-    s.conv(p + ".conv1", planes, inplanes, 1)
-    s.bn(p + ".bn1", planes)
-    s.conv(p + ".conv2", planes, planes, 3)
-    s.bn(p + ".bn2", planes)
-    s.conv(p + ".conv3", planes * 4, planes, 1)
+def _bottleneck(s: ParamSpec, p, inplanes, planes, downsample, groups=1, base_width=64, se=True):
+    """Bottleneck keys: Cadene SEResNetBottleneck / SEResNeXtBottleneck (se=True) or torchvision Bottleneck
+    (se=False).  conv2 is the 3x3 with ``groups``; width = floor(planes * base_width / 64) * groups (planes for
+    the SE-ResNet and ResNet-50 blocks); the 1x1 downsample (kernel 1, padding 0) follows the block's own modules."""
+    width = planes * base_width // 64 * groups
+    s.conv(p + ".conv1", width, inplanes, 1)
+    s.bn(p + ".bn1", width)
+    s.conv(p + ".conv2", width, width // groups, 3)
+    s.bn(p + ".bn2", width)
+    s.conv(p + ".conv3", planes * 4, width, 1)
     s.bn(p + ".bn3", planes * 4)
-    s.conv(p + ".se_module.fc1", planes * 4 // 16, planes * 4, 1, bias=True)
-    s.conv(p + ".se_module.fc2", planes * 4, planes * 4 // 16, 1, bias=True)
+    if se:
+        s.conv(p + ".se_module.fc1", planes * 4 // 16, planes * 4, 1, bias=True)
+        s.conv(p + ".se_module.fc2", planes * 4, planes * 4 // 16, 1, bias=True)
     if downsample:
         s.conv(p + ".downsample.0", planes * 4, inplanes, 1)
         s.bn(p + ".downsample.1", planes * 4)
 
 
-def _senet_layers(s: ParamSpec, p, n_layers: int):
+_LAYERS_50 = ((64, 3), (128, 4), (256, 6), (512, 3))
+
+
+def _senet_layers(s: ParamSpec, p, n_layers: int, groups=1, base_width=64):
+    """Cadene SENet encoder: se_resnet50 (groups 1) or se_resnext50_32x4d (groups 32, base_width 4)."""
     s.conv(p + ".layer0.conv1", 64, 3, 7)
     s.bn(p + ".layer0.bn1", 64)
     inplanes = 64
-    for li, (planes, blocks) in enumerate(((64, 3), (128, 4), (256, 6), (512, 3))[:n_layers], start=1):
+    for li, (planes, blocks) in enumerate(_LAYERS_50[:n_layers], start=1):
         for b in range(blocks):
-            _se_bottleneck(s, f"{p}.layer{li}.{b}", inplanes, planes, downsample=(b == 0))
+            _bottleneck(s, f"{p}.layer{li}.{b}", inplanes, planes, b == 0, groups, base_width)
+            inplanes = planes * 4
+
+
+def _resnet50(s: ParamSpec, p, groups=1, base_width=64):
+    """torchvision ResNet-50 / ResNeXt-50 as smp's ResNetEncoder keeps it (no fc)."""
+    s.conv(p + ".conv1", 64, 3, 7)
+    s.bn(p + ".bn1", 64)
+    inplanes = 64
+    for li, (planes, blocks) in enumerate(_LAYERS_50, start=1):
+        for b in range(blocks):
+            _bottleneck(s, f"{p}.layer{li}.{b}", inplanes, planes, b == 0, groups, base_width, se=False)
             inplanes = planes * 4
 
 
@@ -153,6 +173,16 @@ def _resnet34(s: ParamSpec, p):
                 s.conv(q + ".downsample.0", planes, inplanes, 1)
                 s.bn(q + ".downsample.1", planes)
             inplanes = planes
+
+
+#: smp 0.1.3 encoder names on the hot path -> parameter layout under "encoder."
+SMP_ENCODERS = {
+    "resnet34": _resnet34,
+    "resnet50": _resnet50,
+    "resnext50_32x4d": lambda s, p: _resnet50(s, p, groups=32, base_width=4),
+    "se_resnet50": lambda s, p: _senet_layers(s, p, 4),
+    "se_resnext50_32x4d": lambda s, p: _senet_layers(s, p, 4, groups=32, base_width=4),
+}
 
 
 # ------------------------------------------------------------------- decoders
@@ -226,14 +256,10 @@ def build_unetplusplusstar(s: ParamSpec, base_dim=32, decoder_attention_type="sc
 
 def build_smp_style(s: ParamSpec, encoder_name, decoder="unetplusplus", decoder_attention_type=None, classes=1,
                     decoder_use_batchnorm=True, deep_heads=False):
-    if encoder_name == "se_resnet50":
-        _senet_layers(s, "encoder", 4)
-        enc_ch = (3, 64, 256, 512, 1024, 2048)
-    elif encoder_name == "resnet34":
-        _resnet34(s, "encoder")
-        enc_ch = (3, 64, 64, 128, 256, 512)
-    else:
-        raise KeyError(f"encoder {encoder_name!r} is outside the B200 hot path (resnet34, se_resnet50)")
+    if encoder_name not in SMP_ENCODERS:
+        raise KeyError(f"encoder {encoder_name!r} is outside the B200 hot path ({', '.join(SMP_ENCODERS)})")
+    SMP_ENCODERS[encoder_name](s, "encoder")
+    enc_ch = (3, 64, 64, 128, 256, 512) if encoder_name == "resnet34" else (3, 64, 256, 512, 1024, 2048)
     if decoder == "unetplusplus":
         blocks = [(n, i, s_, o) for n, _, i, s_, o in dense_decoder_blocks(enc_ch)]
     else:  # smp Unet

@@ -17,6 +17,9 @@
 //   B tile : TMA box [block_k][block_n] of the [Cout][taps*C] weight matrix.
 //   D      : 128 TMEM lanes x block_n fp32 columns, two buffers (epilogue of tile t overlaps tile t+1).
 //   A second input map can follow the first along K (decoder concat read as two dense maps).
+//   Grouped mode (ResNeXt 3x3, 64 % channels-per-group == 0): block_n = block_k = 64 and cout tile n reads only
+//            input chunk n, so the K loop is the taps alone; the A box starts at channel n * 64 (a_nt_ch) and B is a
+//            block-diagonal [Cout][taps][64] matrix (zeros outside each output channel's group).
 // Persistent: grid = min(#tiles, #SMs), the TMA ring runs across tile boundaries.
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
 // warps 2-9 = epilogue (TMEM -> registers -> bias/residual/ReLU -> bf16 -> swizzled shared memory ->
@@ -39,6 +42,7 @@ struct IgemmParams {
     CUtensorMap a_map[4];
     CUtensorMap a_map1;     // optional second input (channels C0.. of the concatenated K axis), stride 1 only
     int k_split;            // channel chunks served by a_map (== k_chunks when there is one input)
+    int a_nt_ch;            // input channels the A box advances per cout tile: 64 in grouped mode, 0 when dense
     CUtensorMap b_map;
     const float* bias;
     const float* gate;      // optional [N][Cout]: y = relu((acc + bias) * gate[n][co] + residual)  (SE scale fused)
@@ -126,7 +130,7 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                     uint8_t* sa = smem + (size_t)stage * stage_bytes;
                     uint8_t* sb = sa + p.a_stage_bytes;
                     if (kc < p.k_split)
-                        tma_load_4d(sa, &p.a_map[p.tap_plane[tap]], &full_bar[stage], kc * p.block_k,
+                        tma_load_4d(sa, &p.a_map[p.tap_plane[tap]], &full_bar[stage], kc * p.block_k + n_tile * p.a_nt_ch,
                                     w0 + p.tap_dw[tap], h0 + p.tap_dh[tap], n0);
                     else
                         tma_load_4d(sa, &p.a_map1, &full_bar[stage], (kc - p.k_split) * p.block_k,
@@ -425,9 +429,10 @@ int tmap_encode_bf16(CUtensorMap* map, const void* base, int rank, const cuuint6
 using namespace eds;
 
 // x: [N][H][W][C0]; x1 (optional): [N][H][W][C1] -- the convolution of their channel concatenation
+// groups > 1: grouped convolution, w the block-diagonal [Cout][R][S][64] matrix (eds_conv2d_igemm_grouped_supported)
 static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, int H, int W, const void* w,
                         const float* bias, int Cout, int R, int S, int stride, int pad, int relu, const void* residual,
-                        void* y, void* stream, const float* gate = nullptr) {
+                        void* y, void* stream, const float* gate = nullptr, int groups = 1) {
     const int C = C0 + C1;
     EDS_REQUIRE(x && w && y, "conv2d_igemm: null pointer");
     EDS_REQUIRE(N > 0 && H > 0 && W > 0, "conv2d_igemm: bad shape N=%d H=%d W=%d", N, H, W);
@@ -458,11 +463,17 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     p.block_k = ((C0 | C1) % 64 == 0) ? 64 : ((C0 | C1) % 32 == 0 ? 32 : 16);   // divides both inputs
     p.k_chunks = C / p.block_k;
     p.k_split = C0 / p.block_k;
-    const int k_iters = p.taps * p.k_chunks;
     // cout tile: the largest multiple of 16 that divides Cout and is <= 256 (two accumulators of
     // block_n fp32 columns fit the 512 columns of TMEM)
     int bn = 256;
     while (bn > 16 && Cout % bn != 0) bn -= 16;
+    if (groups > 1) {        // one 64-channel input chunk per 64-channel cout tile; B rows are taps x 64 wide
+        p.C = 64;
+        p.k_chunks = p.k_split = 1;
+        p.a_nt_ch = 64;
+        bn = 64;
+    }
+    const int k_iters = p.taps * p.k_chunks;
     p.block_n = bn;
     p.n_tiles = Cout / bn;
     p.N = N; p.Ho = Ho; p.Wo = Wo; p.Cout = Cout; p.relu = relu;
@@ -563,8 +574,8 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     }
     if (!plane_used[0]) p.a_map[0] = p.a_map[p.tap_plane[0]];  // keep the prefetch target valid
     {
-        cuuint64_t dims[2] = {(cuuint64_t)p.taps * C, (cuuint64_t)Cout};
-        cuuint64_t strides[1] = {(cuuint64_t)p.taps * C * 2};
+        cuuint64_t dims[2] = {(cuuint64_t)p.taps * p.C, (cuuint64_t)Cout};
+        cuuint64_t strides[1] = {(cuuint64_t)p.taps * p.C * 2};
         cuuint32_t box[2] = {(cuuint32_t)p.block_k, (cuuint32_t)p.block_n};
         if (int rc = tmap_encode_bf16(&p.b_map, w, 2, dims, strides, box, swz, "weights")) return rc;
     }
@@ -599,4 +610,22 @@ extern "C" int eds_conv2d_igemm_bf16_2src(const void* x0, int C0, const void* x1
                                           const void* residual, void* y, void* stream) {
     EDS_REQUIRE(x1 && C1 > 0, "conv2d_igemm_2src: second input missing");
     return igemm_launch(x0, C0, x1, C1, N, H, W, w, bias, Cout, R, S, 1, pad, relu, residual, y, stream);
+}
+
+extern "C" int eds_conv2d_igemm_grouped_supported(int C, int Cout, int groups, int R, int S, int stride) {
+    if (groups < 2 || C <= 0 || C % groups != 0 || C != Cout || C % 64 != 0) return 0;
+    const int cpg = C / groups;
+    return 64 % cpg == 0 && R == S && (R == 1 || R == 3) && (stride == 1 || stride == 2);
+}
+
+extern "C" int eds_conv2d_igemm_bf16_grouped(const void* x, int N, int H, int W, int C, const void* w_packed,
+                                             const float* bias, int groups, int Cout, int R, int S, int stride, int pad,
+                                             int relu, const void* residual, void* y, void* stream) {
+    EDS_REQUIRE(groups >= 2 && C > 0 && C % groups == 0 && 64 % (C / groups) == 0,
+                "conv2d_igemm_grouped: C=%d groups=%d: the channels per group must divide 64", C, groups);
+    EDS_REQUIRE(C == Cout && C % 64 == 0, "conv2d_igemm_grouped: C=%d Cout=%d must be equal multiples of 64", C, Cout);
+    EDS_REQUIRE(eds_conv2d_igemm_grouped_supported(C, Cout, groups, R, S, stride),
+                "conv2d_igemm_grouped: filter %dx%d stride %d not supported (1x1, 3x3; stride 1, 2)", R, S, stride);
+    return igemm_launch(x, C, nullptr, 0, N, H, W, w_packed, bias, Cout, R, S, stride, pad, relu, residual, y, stream,
+                        nullptr, groups);
 }

@@ -4,6 +4,7 @@
 // as the independent cross-check of the tensor-core kernel in tests/.  It is not a
 // fallback: the bf16 product path never dispatches here.
 #include "common.cuh"
+#include <algorithm>
 
 namespace eds {
 
@@ -104,9 +105,61 @@ conv_simt_kernel(const T* __restrict__ x, int N, int H, int W, int C, const T* _
     }
 }
 
+// Grouped convolution (ResNeXt 3x3, fp32 parity mode): one thread per output element, channel fastest so a warp's
+// stores and weight reads are contiguous; the reduction (taps x channels of the group, in that order) is one fp32 fma
+// chain.  w: [Cout][R][S][C / groups].
+template <typename T>
+__global__ void __launch_bounds__(256)
+conv_simt_grouped_kernel(const T* __restrict__ x, int N, int H, int W, int C, const T* __restrict__ w,
+                         const float* __restrict__ bias, int cpg, int Cout, int R, int S, int stride, int pad, int Ho,
+                         int Wo, int relu, const T* __restrict__ residual, T* __restrict__ y) {
+    const int64_t total = (int64_t)N * Ho * Wo * Cout;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int co = (int)(i % Cout);
+        const int64_t m = i / Cout;
+        const int ow = (int)(m % Wo), oh = (int)((m / Wo) % Ho), n = (int)(m / ((int64_t)Wo * Ho));
+        const int c0 = (co / (Cout / (C / cpg))) * cpg;        // first input channel of co's group
+        const T* wr = w + (int64_t)co * R * S * cpg;
+        float acc = 0.f;
+        for (int r = 0; r < R; ++r) {
+            const int iy = oh * stride - pad + r;
+            if (iy < 0 || iy >= H) continue;
+            for (int s = 0; s < S; ++s) {
+                const int ix = ow * stride - pad + s;
+                if (ix < 0 || ix >= W) continue;
+                const T* xp = x + (((int64_t)n * H + iy) * W + ix) * C + c0;
+                const T* wp = wr + (r * S + s) * cpg;
+                for (int c = 0; c < cpg; ++c) acc = fmaf(Elem<T>::ld(xp + c), Elem<T>::ld(wp + c), acc);
+            }
+        }
+        float v = acc + (bias ? bias[co] : 0.f);
+        if (residual) v += Elem<T>::ld(residual + i);
+        if (relu) v = fmaxf(v, 0.f);
+        Elem<T>::st(y + i, v);
+    }
+}
+
 }  // namespace eds
 
 using namespace eds;
+
+extern "C" int eds_conv2d_simt_grouped(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
+                                       int groups, int Cout, int R, int S, int stride, int pad, int relu,
+                                       const void* residual, void* y, int dtype, void* stream) {
+    EDS_REQUIRE(x && w && y, "conv2d_simt_grouped: null pointer");
+    EDS_REQUIRE(N > 0 && H > 0 && W > 0 && C > 0 && Cout > 0, "conv2d_simt_grouped: bad shape");
+    EDS_REQUIRE(groups >= 1 && C % groups == 0 && Cout % groups == 0,
+                "conv2d_simt_grouped: C=%d and Cout=%d must be multiples of groups=%d", C, Cout, groups);
+    EDS_REQUIRE(R >= 1 && S >= 1 && stride >= 1 && pad >= 0, "conv2d_simt_grouped: bad filter geometry");
+    const int Ho = (H + 2 * pad - R) / stride + 1, Wo = (W + 2 * pad - S) / stride + 1;
+    EDS_REQUIRE(Ho > 0 && Wo > 0, "conv2d_simt_grouped: empty output");
+    const int64_t total = (int64_t)N * Ho * Wo * Cout;
+    const unsigned grid = (unsigned)std::min<int64_t>(ceil_div64(total, 256), 148 * 16);
+    EDS_DISPATCH_DTYPE(dtype, T, (conv_simt_grouped_kernel<T><<<grid, 256, 0, as_stream(stream)>>>(
+                                     (const T*)x, N, H, W, C, (const T*)w, bias, C / groups, Cout, R, S, stride, pad,
+                                     Ho, Wo, relu, (const T*)residual, (T*)y)));
+    return check_launch("conv_simt_grouped_kernel");
+}
 
 extern "C" int eds_conv2d_simt(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
                                int Cout, int R, int S, int stride, int pad, int relu, const void* residual,

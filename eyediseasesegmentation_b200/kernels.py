@@ -290,15 +290,33 @@ def conv_out_hw(H: int, W: int, R: int, stride: int, pad: int):
     return (H + 2 * pad - R) // stride + 1, (W + 2 * pad - R) // stride + 1
 
 
+def pack_grouped_weights(w: torch.Tensor) -> torch.Tensor:
+    """Grouped filter w [Cout,R,S,C/groups] (C == Cout, the channels per group dividing 64) -> the block-diagonal
+    [Cout,R,S,64] operand of eds_conv2d_igemm_bf16_grouped: row co holds the 64 input channels of its 64-channel
+    chunk, zero outside co's group.  Same dtype and device as w (pack in fp32, then cast)."""
+    Cout, R, S, cpg = w.shape
+    assert 64 % cpg == 0 and Cout % 64 == 0, (Cout, cpg)
+    packed = torch.zeros((Cout, R, S, 64), dtype=w.dtype, device=w.device)
+    off = (torch.arange(Cout, device=w.device) // cpg * cpg) % 64           # first channel of co's group in its chunk
+    idx = (off.view(Cout, 1) + torch.arange(cpg, device=w.device).view(1, cpg)).view(Cout, 1, 1, cpg)
+    packed.scatter_(3, idx.expand(Cout, R, S, cpg), w)
+    return packed
+
+
 def conv2d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], stride: int = 1, pad: int = 0,
            relu: bool = False, residual: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None,
-           impl: str = "auto", x1: Optional[torch.Tensor] = None) -> torch.Tensor:
+           impl: str = "auto", x1: Optional[torch.Tensor] = None, groups: int = 1) -> torch.Tensor:
     """x [N,H,W,C], w [Cout,R,S,C] (same dtype as x) -> [N,Ho,Wo,Cout].
 
     impl: "tc" = tcgen05 implicit GEMM (bf16 only; picks the generic, halo-reuse or dw-grouped wide-N kernel by
     layer shape), "halo" / "wide" = force that kernel, "simt" = CUDA-core kernel,
     "auto" = tc for bf16 activations, simt for fp32 (the fp32 parity mode).
+
+    groups > 1 (ResNeXt 3x3): always the grouped kernels, w [Cout,R,S,64] from pack_grouped_weights on the tensor
+    cores, w [Cout,R,S,C/groups] on the CUDA cores.  A shape the grouped tcgen05 kernel does not take raises.
     """
+    if groups > 1:
+        return _conv2d_grouped(x, w, bias, groups, stride, pad, relu, residual, out, impl)
     _chk(x, w, bias, residual, out, x1)
     N, H, W_, Cin = x.shape
     Cout, R, S, Cw = w.shape
@@ -366,6 +384,43 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], strid
                                          _p(residual), _p(out), _dt(x), _stream()))
     else:
         raise ValueError(impl)
+    return out
+
+
+def _conv2d_grouped(x, w, bias, groups, stride, pad, relu, residual, out, impl):
+    _chk(x, w, bias, residual, out)
+    N, H, W_, Cin = x.shape
+    Cout, R, S, Cw = w.shape
+    assert w.dtype == x.dtype and Cin % groups == 0
+    Ho, Wo = conv_out_hw(H, W_, R, stride, pad)
+    if out is None:
+        out = torch.empty((N, Ho, Wo, Cout), dtype=x.dtype, device=x.device)
+    if impl == "auto":
+        impl = "tc" if x.dtype == torch.bfloat16 else "simt"
+    if impl == "tc":
+        if x.dtype != torch.bfloat16:
+            raise TypeError("the tcgen05 kernel takes bf16 activations")
+        if not _lib.load().eds_conv2d_igemm_grouped_supported(Cin, Cout, groups, R, S, stride):
+            raise ValueError(f"grouped convolution C={Cin} Cout={Cout} groups={groups} {R}x{S} stride {stride} is not "
+                             "supported by the tcgen05 kernel (C == Cout, C % 64 == 0, C / groups dividing 64)")
+        assert Cw == 64, "tensor-core grouped weights are the packed [Cout,R,S,64] operand (pack_grouped_weights)"
+        trace = CONV_TRACE
+        if trace is not None:
+            ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            ev0.record()
+        _TAG[0] = f"conv_igemm {R}x{R} grouped (tcgen05)"
+        check(_lib.lib().eds_conv2d_igemm_bf16_grouped(_p(x), N, H, W_, Cin, _p(w), _p(bias), groups, Cout, R, S,
+                                                       stride, pad, int(relu), _p(residual), _p(out), _stream()))
+        if trace is not None:
+            ev1.record()
+            trace.append((2.0 * N * Ho * Wo * Cout * R * S * (Cin // groups), ev0, ev1,
+                          (N, H, W_, Cin, Cout, R, stride, groups)))
+    elif impl == "simt":
+        assert Cw == Cin // groups
+        check(_lib.lib().eds_conv2d_simt_grouped(_p(x), N, H, W_, Cin, _p(w), _p(bias), groups, Cout, R, S, stride,
+                                                 pad, int(relu), _p(residual), _p(out), _dt(x), _stream()))
+    else:
+        raise ValueError(f"grouped convolutions run on the grouped tcgen05 or CUDA-core kernel, not {impl!r}")
     return out
 
 

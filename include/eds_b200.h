@@ -198,6 +198,19 @@ EDS_API int eds_conv2d_igemm_bf16_gated(const void* x, int N, int H, int W, int 
                                 const float* bias, const float* gate, int Cout, int R, int S, int stride,
                                 int pad, int relu, const void* residual, void* y, void* stream);
 
+/* Grouped convolution on the same tcgen05 pipeline (ResNeXt 3x3 conv2 with 32 groups: the torchvision Bottleneck
+ * of resnext50_32x4d and the Cadene SEResNeXtBottleneck of se_resnext50_32x4d, both reached through smp 0.1.3's
+ * get_encoder; replaces their cuDNN nn.Conv2d(groups=32)).  C == Cout, C % 64 == 0 and the channels per group
+ * (C / groups) divide 64, so every 64-channel cout tile reads one 64-channel input chunk.  w_packed is the
+ * block-diagonal [Cout][R][S][64] bf16 matrix: row co holds the 64 input channels of co's chunk, zero outside
+ * co's group (BN folded in fp32 before the cast).  Other arguments as eds_conv2d_igemm_bf16.
+ * eds_conv2d_igemm_grouped_supported returns 1 for the shapes the kernel takes; the others are rejected with
+ * an eds_last_error() message. */
+EDS_API int eds_conv2d_igemm_grouped_supported(int C, int Cout, int groups, int R, int S, int stride);
+EDS_API int eds_conv2d_igemm_bf16_grouped(const void* x, int N, int H, int W, int C, const void* w_packed,
+                                          const float* bias, int groups, int Cout, int R, int S, int stride, int pad,
+                                          int relu, const void* residual, void* y, void* stream);
+
 /* out[n][co] = sum_ci w[co][ci] * m[n][ci] + b[co]   (fp32; w [Cout][Cin] row-major, b may be NULL). */
 EDS_API int eds_affine_rows(const float* m, int N, int Cin, const float* w, const float* b, int Cout, float* out,
                     void* stream);
@@ -208,6 +221,13 @@ EDS_API int eds_affine_rows(const float* m, int N, int Cin, const float* w, cons
 EDS_API int eds_conv2d_simt(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
                     int Cout, int R, int S, int stride, int pad, int relu, const void* residual,
                     void* y, int dtype, void* stream);
+
+/* Grouped form of eds_conv2d_simt (fp32 parity mode of the ResNeXt conv2, nn.Conv2d(groups=...)):
+ * w [Cout][R][S][C / groups] in the activation dtype, output channel co reads the input channels of group
+ * co / (Cout / groups).  Any group size. */
+EDS_API int eds_conv2d_simt_grouped(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
+                                    int groups, int Cout, int R, int S, int stride, int pad, int relu,
+                                    const void* residual, void* y, int dtype, void* stream);
 
 /* Segmentation head: 3x3 pad-1 conv C->classes with bias, fp32 logits out
  * ([N][classes][H][W], NCHW like the reference output).  w: [classes][3][3][C] fp32. */
