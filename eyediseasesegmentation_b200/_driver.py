@@ -124,8 +124,6 @@ def fused_blend_views(model, transforms, S: int, dst_w: int):
     canvas width qualify, else None (the drivers then merge and paste with two kernels)."""
     if getattr(model, "forward_tta", None) is None or not tta.is_fusable(transforms):
         return None
-    if os.environ.get("EDS_FUSED_BLEND", "1") == "0":
-        return None
     _, deaug = tta.view_maps(transforms, S, S)
     return deaug if K.tta_blend_supported(len(deaug), S, deaug, dst_w) else None
 

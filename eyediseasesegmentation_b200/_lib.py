@@ -62,7 +62,7 @@ PROTOTYPES = {
     "eds_conv3x3_halo_supported": [_i, _i, _i, _i, _i, _i],
     "eds_conv3x3_halo_bf16": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp, _vp],
     "eds_conv3x3_small_supported": [_i, _i],
-    "eds_conv3x3_small_bf16": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
+    "eds_conv3x3_small_bf16": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _vp, _vp],
     "eds_conv2d_simt": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp],
     "eds_conv2d_simt_grouped": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _vp],
     "eds_head_conv3x3": [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _i, _vp],

@@ -24,10 +24,9 @@ from .. import _lib, kernels as K
 from .spec import dense_decoder_blocks
 
 IDENTITY_VIEW = [(1, 0, 0, 0, 1, 0)]
-#: SE bottleneck tail (squeeze, scale, residual, ReLU) in conv3's epilogue on the tensor-core path
-#: (EDS_SE_EPILOGUE=0 keeps conv3 -> channel_mean -> se_gate -> se_scale_add_relu as separate passes)
-SE_IN_EPILOGUE = __import__("os").environ.get("EDS_SE_EPILOGUE", "1") != "0"
-SE_EPILOGUE_MIN_PIXELS = int(__import__("os").environ.get("EDS_SE_EPILOGUE_MIN_PIXELS", str(256 * 256)))
+#: on the tensor-core path, SE bottleneck maps of at least this many pixels get the block's tail (scale, residual,
+#: ReLU) in conv3's epilogue; smaller ones run conv3 and se_scale_add_relu as separate passes
+SE_EPILOGUE_MIN_PIXELS = 256 * 256
 BN_EPS = 1e-5
 
 
@@ -338,7 +337,7 @@ class Engine:
         out = self._cv(x, p + ".conv1", stride=s1, relu=True)
         out = self._cv(out, p + ".conv2", stride=s2, pad=1, relu=True)
         res = self._cv(x, p + ".downsample", stride=stride) if (p + ".downsample") in self.w else x
-        if self.conv_impl == "tc" and SE_IN_EPILOGUE:
+        if self.conv_impl == "tc":
             # conv3 (1x1 + folded BN) has no activation, so the channel means its SE module squeezes are an affine
             # function of the channel means of conv3's INPUT (a quarter of the channels): the gate is known before
             # conv3 runs and the squeeze never re-reads the 4x wider map.  On the large maps scale + residual + ReLU
@@ -446,20 +445,11 @@ class Engine:
         else:
             if skips and (p + ".attention1.sse") in self.w:
                 cat = self._concat_scse(p + ".attention1", x, skips, skip_names)
-            elif (not skips and self.conv_impl == "tc" and K.FUSED_TAIL and
-                  _lib.load().eds_conv3x3_small_supported(x.shape[3], self.w[p + ".conv1"][0].shape[0])):
-                # last block: no skip, no attention1 -- upsampling (and the pending gate of x) is fused into
-                # conv1's tile loader, the upsampled map is never written
-                t, cg, sg = _parts(x)
-                w1, b1 = self.w[p + ".conv1"]
-                cat = None
-                y = K.conv3x3_small(t, w1, b1, True, self.up_mode, cg, sg)
             else:
                 srcs = [_parts(x)] + [_parts(t) for t in skips]
                 cat = K.concat_gated_split(srcs, self.up_mode) if self._split_ok(srcs) else \
                     K.concat_gated(srcs, self.up_mode)
-        if cat is not None:
-            y = self._cv(cat, p + ".conv1", pad=1, relu=True)
+        y = self._cv(cat, p + ".conv1", pad=1, relu=True)
         y = self._cv(y, p + ".conv2", pad=1, relu=True)
         if (p + ".down_sample") not in self.w:
             y = self._apply_scse(p + ".attention2", y)

@@ -12,7 +12,6 @@
 // One CTA handles one (sequence, head); sequences are rows or columns of the NHWC map,
 // addressed by stride so no rearrange / permute is ever materialised.
 #include "common.cuh"
-#include <cstdlib>
 
 namespace eds {
 
@@ -135,9 +134,8 @@ extern "C" int eds_axial_attention(const void* qk, int qk_cstride, const void* v
     EDS_REQUIRE(axis == 0 || axis == 1, "axial_attention: axis=%d", axis);
     EDS_REQUIRE(N > 0 && H > 0 && W > 0 && heads > 0 && dqk > 0 && dv > 0, "axial_attention: bad shape");
     // bf16 activations: tensor-core kernel (attention_mma.cu); fp32 parity mode and shapes outside it
-    // (dqk != 8, heads % 4 != 0, L > 64) run the CUDA-core kernel below.  EDS_ATTN_SIMT=1 forces the latter.
-    static const bool force_simt = getenv("EDS_ATTN_SIMT") && atoi(getenv("EDS_ATTN_SIMT")) != 0;
-    if (dtype == EDS_BF16 && !force_simt) {
+    // (dqk != 8, heads % 4 != 0, L > 64) run the CUDA-core kernel below.
+    if (dtype == EDS_BF16) {
         const int rc = axial_attention_mma_try(qk, qk_cstride, v, v_cstride, N, H, W, axis, heads, dqk, dv, rel,
                                                sim_scale, out_scale, out_shift, relu, y, as_stream(stream));
         if (rc <= 0) return rc;

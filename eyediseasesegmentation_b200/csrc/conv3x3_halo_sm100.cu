@@ -22,7 +22,6 @@
 // Tiles are walked round-robin (tile = blockIdx.x + i * gridDim.x), grid = min(#tiles, #SMs).
 #include "tc_ptx.cuh"
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -45,7 +44,6 @@ struct HaloParams {
     int tiles_w, tiles_h, total_tiles;
     int stages, atom_bytes, a_slab_bytes, b_tap_bytes, stage_bytes, tmem_cols;
     uint32_t idesc, desc_hi;
-    int debug;   // developer timing switches (EDS_HALO_DEBUG): 1 = no TMA issue, 2 = no MMA issue
 };
 
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
@@ -98,22 +96,18 @@ conv3x3_halo_kernel(const __grid_constant__ HaloParams p) {
                 for (int kc = 0; kc < p.k_chunks; ++kc)
                     for (int dwi = 0; dwi < 3; ++dwi) {
                         mbar_wait(&empty_bar[stage], phase ^ 1u);
-                        if (p.debug & 1) {
-                            mbar_arrive(&full_bar[stage]);
-                        } else {
-                            mbar_arrive_expect_tx(&full_bar[stage],
-                                                  (uint32_t)((kSlabRows * p.atom_bytes) + 3 * p.bn * p.block_k * 2));
-                            uint8_t* sa = smem + (size_t)stage * p.stage_bytes;
-                            uint8_t* sb = sa + p.a_slab_bytes;
-                            if (kc < p.k_split)
-                                tma_load_4d(sa, &p.a_map, &full_bar[stage], kc * p.block_k, w0 + dwi - 1, h0 - 1, n);
-                            else
-                                tma_load_4d(sa, &p.a_map1, &full_bar[stage], (kc - p.k_split) * p.block_k, w0 + dwi - 1,
-                                            h0 - 1, n);
-                            for (int dhi = 0; dhi < 3; ++dhi)
-                                tma_load_2d(sb + dhi * p.b_tap_bytes, &p.b_map, &full_bar[stage],
-                                            (dhi * 3 + dwi) * p.C + kc * p.block_k, 0);
-                        }
+                        mbar_arrive_expect_tx(&full_bar[stage],
+                                              (uint32_t)((kSlabRows * p.atom_bytes) + 3 * p.bn * p.block_k * 2));
+                        uint8_t* sa = smem + (size_t)stage * p.stage_bytes;
+                        uint8_t* sb = sa + p.a_slab_bytes;
+                        if (kc < p.k_split)
+                            tma_load_4d(sa, &p.a_map, &full_bar[stage], kc * p.block_k, w0 + dwi - 1, h0 - 1, n);
+                        else
+                            tma_load_4d(sa, &p.a_map1, &full_bar[stage], (kc - p.k_split) * p.block_k, w0 + dwi - 1,
+                                        h0 - 1, n);
+                        for (int dhi = 0; dhi < 3; ++dhi)
+                            tma_load_2d(sb + dhi * p.b_tap_bytes, &p.b_map, &full_bar[stage],
+                                        (dhi * 3 + dwi) * p.C + kc * p.block_k, 0);
                         if (++stage == p.stages) { stage = 0; phase ^= 1u; }
                     }
             }
@@ -136,7 +130,7 @@ conv3x3_halo_kernel(const __grid_constant__ HaloParams p) {
             for (int it = 0; it < iters_per_tile; ++it) {
                 mbar_wait(&full_bar[stage], phase);
                 tc_fence_after();
-                if (elect_one() && !(p.debug & 2)) {
+                if (elect_one()) {
                     const uint32_t a_st = lo0 + (uint32_t)stage * stage16, b_st = a_st + slab16;
                     const uint32_t acc0 = it > 0 ? 1u : 0u;
 #pragma unroll
@@ -235,7 +229,6 @@ conv3x3_halo_kernel(const __grid_constant__ HaloParams p) {
 
 static PerDevice g_halo_once;             // the shared-memory opt-in belongs to a device's context
 static int g_num_sms = 148;
-static int g_stage_override = 0;
 
 static int halo_init() {
     return g_halo_once.run([](int dev) {
@@ -287,13 +280,10 @@ static int halo_launch(const void* x, int C0, const void* x1, int C1, int N, int
     p.y = (__nv_bfloat16*)y;
     p.C = C;
     p.block_k = ((C0 | C1) % 64 == 0) ? 64 : ((C0 | C1) % 32 == 0 ? 32 : 16);   // divides both inputs
-    if (const char* bk = getenv("EDS_HALO_BK")) { const int v = atoi(bk); if ((v == 32 || v == 16) && (C0 | C1) % v == 0) p.block_k = std::min(p.block_k, v); }
     p.k_chunks = C / p.block_k;
     p.k_split = C0 / p.block_k;
     p.bn = Cout;
     p.N = N; p.H = H; p.W = W; p.relu = relu;
-    if (const char* dbg = getenv("EDS_HALO_DEBUG")) p.debug = atoi(dbg);
-    if (const char* st = getenv("EDS_HALO_STAGES")) g_stage_override = atoi(st);
     p.tiles_w = ceil_div(W, kTileCols);
     p.tiles_h = ceil_div(H, kTileRows);
     const int64_t total = (int64_t)p.tiles_w * p.tiles_h * N;
@@ -311,7 +301,6 @@ static int halo_launch(const void* x, int C0, const void* x1, int C1, int N, int
     p.b_tap_bytes = (p.bn * p.block_k * 2 + 1023) & ~1023;
     p.stage_bytes = p.a_slab_bytes + 3 * p.b_tap_bytes;
     p.stages = std::max(2, std::min(kHaloStagesMax, (200 * 1024) / p.stage_bytes));
-    if (g_stage_override > 0) p.stages = std::min(p.stages, g_stage_override);
     p.tmem_cols = std::max(32, pow2_ceil_i(4 * p.bn));
     const size_t smem = (size_t)p.stages * p.stage_bytes + 1024 + (2 * kHaloStagesMax + 4) * 8 + 16;
     EDS_REQUIRE(smem <= 227 * 1024 && p.tmem_cols <= 512, "conv3x3_halo: tile does not fit (smem %zu, tmem %d)", smem,

@@ -1,17 +1,11 @@
-// 3x3 / stride 1 / pad 1 convolution for the full-resolution tail of the decoders (Cin, Cout in {16, 32}),
-// optionally fused with the x2 upsampling of a GATED low-resolution input.
+// 3x3 / stride 1 / pad 1 convolution for the full-resolution tail of the decoders (Cin = 16, Cout in {16, 32}).
 //
-// Reference: the last decoder block (x_0_4 of unetplusplusstar.py:239-263 / DecoderBlock.forward :151-161; block 4
-// of smp.Unet): x = interpolate(x, 2) -> conv1 (32 -> 16) + BN + ReLU -> conv2 (16 -> 16) + BN + ReLU, and the
-// 32 -> 32 conv2 of the block before.  At 1024^2 these layers hold 0.8 % of the network's FLOPs but every
-// intermediate is a 1.6 - 3.2 GB map (48-map batch): they are bound by bytes, and a 16-column tcgen05 tile
-// wastes the 128 x N datapath (measured 100 - 240 TFLOP/s in the implicit-GEMM kernels).  Here one CTA owns a
-// 16 x 32 pixel output tile:
-//   1. the 18 x 34 input halo tile is built in shared memory as bf16 -- read directly, or (UP) computed on
-//      the fly from the low-resolution map: pending SCSE gate (cgate[n][c] + sgate[n][p]) applied to each
-//      low-res pixel, then bilinear (align_corners=False) / nearest x2 -- so the upsampled 3.2 GB map of the
-//      first version is never written or read;
-//   2. 8 warps x (2 rows x 32 px) x Cout x (9 taps x Cin) as mma.sync.m16n8k16 straight from that tile
+// Reference: conv2 (16 -> 16) + BN + ReLU of the last decoder block (x_0_4 of unetplusplusstar.py:239-263 /
+// DecoderBlock.forward :151-161; block 4 of smp.Unet).  At 1024^2 such a layer holds a fraction of a percent of the
+// network's FLOPs but its input and output are 1.6 GB maps each (48-map batch): it is bound by bytes, and a
+// 16-column tcgen05 tile wastes the 128 x N datapath (measured 100 - 240 TFLOP/s in the implicit-GEMM kernels).  Here one CTA owns a 16 x 32 pixel output tile:
+//   1. the 18 x 34 input halo tile is copied to shared memory as bf16;
+//   2. 8 warps x (2 rows x 32 px) x Cout x (9 taps x 16 channels) as mma.sync.m16n8k16 straight from that tile
 //      (im2col is only an address: row = pixel, k = (tap, channel));
 //   3. bias + ReLU -> bf16 -> staging tile -> 16-byte coalesced stores.
 #include "common.cuh"
@@ -20,12 +14,10 @@ namespace eds {
 
 constexpr int kSmallTH = 16, kSmallTW = 32;                  // output tile
 constexpr int kSmallHH = kSmallTH + 2, kSmallHW = kSmallTW + 2;
-
-template <int CIN> struct SmallCfg {
-    static constexpr int PS = CIN + 8;                       // bf16 per halo pixel (bank-conflict-free fragments)
-    static constexpr int KP = 9 * CIN + 8;                   // bf16 per weight row
-    static constexpr size_t in_bytes = (size_t)kSmallHH * kSmallHW * PS * 2;
-};
+constexpr int kSmallCin = 16;
+constexpr int kSmallPS = kSmallCin + 8;                      // bf16 per halo pixel (bank-conflict-free fragments)
+constexpr int kSmallKP = 9 * kSmallCin + 8;                  // bf16 per weight row
+constexpr size_t kSmallInBytes = (size_t)kSmallHH * kSmallHW * kSmallPS * 2;
 
 __device__ __forceinline__ void small_mma(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
                                           uint32_t b1) {
@@ -35,17 +27,15 @@ __device__ __forceinline__ void small_mma(float (&c)[4], uint32_t a0, uint32_t a
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-// UP: 0 = x is [N][H][W][CIN]; 1 = x is [N][H/2][W/2][CIN], nearest x2; 2 = bilinear x2 (align_corners=False)
-template <int CIN, int COUT, int UP>
+// x [N][H][W][16], wgt [COUT][3][3][16] -> y [N][H][W][COUT]
+template <int COUT>
 __global__ void __launch_bounds__(256)
-conv3x3_small_kernel(const __nv_bfloat16* __restrict__ x, const float* __restrict__ cgate,
-                     const float* __restrict__ sgate, int H, int W, const __nv_bfloat16* __restrict__ wgt,
+conv3x3_small_kernel(const __nv_bfloat16* __restrict__ x, int H, int W, const __nv_bfloat16* __restrict__ wgt,
                      const float* __restrict__ bias, int relu, __nv_bfloat16* __restrict__ y) {
-    using Cfg = SmallCfg<CIN>;
-    constexpr int PS = Cfg::PS, KP = Cfg::KP, NT = COUT / 8, KC = CIN / 16, V8N = CIN / 8;
+    constexpr int CIN = kSmallCin, PS = kSmallPS, KP = kSmallKP, NT = COUT / 8, KC = CIN / 16, V8N = CIN / 8;
     extern __shared__ __align__(16) uint8_t sm_raw[];
     __nv_bfloat16* s_in = reinterpret_cast<__nv_bfloat16*>(sm_raw);                        // [18][34][PS]
-    __nv_bfloat16* s_w = reinterpret_cast<__nv_bfloat16*>(sm_raw + ((Cfg::in_bytes + 15) & ~(size_t)15));   // [COUT][KP]
+    __nv_bfloat16* s_w = reinterpret_cast<__nv_bfloat16*>(sm_raw + ((kSmallInBytes + 15) & ~(size_t)15));   // [COUT][KP]
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int n = blockIdx.z;
     const int oy0 = blockIdx.y * kSmallTH, ox0 = blockIdx.x * kSmallTW;
@@ -62,56 +52,7 @@ conv3x3_small_kernel(const __nv_bfloat16* __restrict__ x, const float* __restric
         const int iy = oy0 - 1 + hy, ix = ox0 - 1 + hx;               // coordinates in the conv input (H x W)
         const bool inside = iy >= 0 && iy < H && ix >= 0 && ix < W;   // outside = the convolution's zero padding
         float2 v[4];
-        if (UP == 0) {
-            V8<__nv_bfloat16>::ld(x + (((int64_t)n * H + min(max(iy, 0), H - 1)) * W + min(max(ix, 0), W - 1)) * CIN + v8 * 8, v);
-            if (cgate) {
-                float2 cg[4];
-                ld8f(cgate + (int64_t)n * CIN + v8 * 8, cg);
-                const float2 s2 = f2(__ldg(sgate + ((int64_t)n * H + min(max(iy, 0), H - 1)) * W + min(max(ix, 0), W - 1)));
-#pragma unroll
-                for (int q = 0; q < 4; ++q) v[q] = __fmul2_rn(v[q], __fadd2_rn(cg[q], s2));
-            }
-        } else {
-            const int h = H / 2, w = W / 2;
-            const int cy = min(max(iy, 0), H - 1), cx = min(max(ix, 0), W - 1);
-            const __nv_bfloat16* xb = x + (int64_t)n * h * w * CIN + v8 * 8;
-            const float* sb = sgate ? sgate + (int64_t)n * h * w : nullptr;
-            float2 cg[4];
-            if (cgate) ld8f(cgate + (int64_t)n * CIN + v8 * 8, cg);
-            auto tap = [&](int py, int px, float2 (&o)[4]) {
-                V8<__nv_bfloat16>::ld(xb + (int64_t)(py * w + px) * CIN, o);
-                if (cgate) {
-                    const float2 s2 = f2(__ldg(sb + py * w + px));
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) o[q] = __fmul2_rn(o[q], __fadd2_rn(cg[q], s2));
-                }
-            };
-            if (UP == 1) {
-                tap(cy >> 1, cx >> 1, v);
-            } else {
-                int y0, y1, x0, x1;
-                float ly, lx;
-                const int jy = cy >> 1, jx = cx >> 1;
-                if (cy & 1) { y0 = jy; y1 = min(jy + 1, h - 1); ly = 0.25f; }
-                else if (jy == 0) { y0 = 0; y1 = 0; ly = 0.f; }
-                else { y0 = jy - 1; y1 = jy; ly = 0.75f; }
-                if (cx & 1) { x0 = jx; x1 = min(jx + 1, w - 1); lx = 0.25f; }
-                else if (jx == 0) { x0 = 0; x1 = 0; lx = 0.f; }
-                else { x0 = jx - 1; x1 = jx; lx = 0.75f; }
-                float2 a[4], b[4], c[4], d[4];
-                tap(y0, x0, a);
-                tap(y0, x1, b);
-                tap(y1, x0, c);
-                tap(y1, x1, d);
-                const float2 hx2 = f2(1.f - lx), lx2 = f2(lx), hy2 = f2(1.f - ly), ly2 = f2(ly);
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float2 top = __ffma2_rn(lx2, b[q], __fmul2_rn(hx2, a[q]));
-                    const float2 bot = __ffma2_rn(lx2, d[q], __fmul2_rn(hx2, c[q]));
-                    v[q] = __ffma2_rn(ly2, bot, __fmul2_rn(hy2, top));
-                }
-            }
-        }
+        V8<__nv_bfloat16>::ld(x + (((int64_t)n * H + min(max(iy, 0), H - 1)) * W + min(max(ix, 0), W - 1)) * CIN + v8 * 8, v);
         if (!inside) {
 #pragma unroll
             for (int q = 0; q < 4; ++q) v[q] = f2(0.f);
@@ -183,19 +124,18 @@ conv3x3_small_kernel(const __nv_bfloat16* __restrict__ x, const float* __restric
     }
 }
 
-template <int CIN, int COUT, int UP>
-static int small_launch(const void* x, const float* cgate, const float* sgate, int N, int H, int W, const void* w,
-                        const float* bias, int relu, void* y, cudaStream_t stream) {
-    using Cfg = SmallCfg<CIN>;
-    const size_t smem_mma = ((Cfg::in_bytes + 15) & ~(size_t)15) + (size_t)COUT * Cfg::KP * 2;
+template <int COUT>
+static int small_launch(const void* x, int N, int H, int W, const void* w, const float* bias, int relu, void* y,
+                        cudaStream_t stream) {
+    const size_t smem_mma = ((kSmallInBytes + 15) & ~(size_t)15) + (size_t)COUT * kSmallKP * 2;
     const size_t smem_out = (size_t)kSmallTH * kSmallTW * (COUT + 8) * 2;      // staging reuses the same space
     const size_t smem = smem_mma > smem_out ? smem_mma : smem_out;
     static PerDevice once;                    // one flag per template instance and per device
     if (smem > 48 * 1024)
-        if (int rc = smem_opt_in(once, conv3x3_small_kernel<CIN, COUT, UP>, (int)smem, "conv3x3_small")) return rc;
+        if (int rc = smem_opt_in(once, conv3x3_small_kernel<COUT>, (int)smem, "conv3x3_small")) return rc;
     dim3 grid(ceil_div(W, kSmallTW), ceil_div(H, kSmallTH), N);
-    conv3x3_small_kernel<CIN, COUT, UP><<<grid, 256, smem, stream>>>(
-        (const __nv_bfloat16*)x, cgate, sgate, H, W, (const __nv_bfloat16*)w, bias, relu, (__nv_bfloat16*)y);
+    conv3x3_small_kernel<COUT><<<grid, 256, smem, stream>>>((const __nv_bfloat16*)x, H, W, (const __nv_bfloat16*)w,
+                                                            bias, relu, (__nv_bfloat16*)y);
     return check_launch("conv3x3_small_kernel");
 }
 
@@ -204,30 +144,18 @@ static int small_launch(const void* x, const float* cgate, const float* sgate, i
 using namespace eds;
 
 extern "C" int eds_conv3x3_small_supported(int C, int Cout) {
-    return (C == 16 || C == 32) && (Cout == 16 || Cout == 32);
+    return C == kSmallCin && (Cout == 16 || Cout == 32);
 }
 
-extern "C" int eds_conv3x3_small_bf16(const void* x, const float* cgate, const float* sgate, int up_mode, int N, int H,
-                                      int W, int C, const void* w, const float* bias, int Cout, int relu, void* y,
-                                      void* stream) {
+extern "C" int eds_conv3x3_small_bf16(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
+                                      int Cout, int relu, void* y, void* stream) {
     EDS_REQUIRE(x && w && y, "conv3x3_small: null pointer");
-    EDS_REQUIRE((cgate == nullptr) == (sgate == nullptr), "conv3x3_small: cgate and sgate come together");
-    EDS_REQUIRE(eds_conv3x3_small_supported(C, Cout), "conv3x3_small: C=%d Cout=%d (16 / 32 only)", C, Cout);
-    EDS_REQUIRE(up_mode == EDS_UP_NONE || up_mode == EDS_UP_NEAREST || up_mode == EDS_UP_BILINEAR,
-                "conv3x3_small: bad up_mode %d", up_mode);
+    EDS_REQUIRE(eds_conv3x3_small_supported(C, Cout), "conv3x3_small: C=%d Cout=%d (C = 16, Cout = 16 / 32 only)", C,
+                Cout);
     EDS_REQUIRE(N > 0 && N <= 65535 && H > 0 && W > 0, "conv3x3_small: bad shape");
-    EDS_REQUIRE(up_mode == EDS_UP_NONE || (H % 2 == 0 && W % 2 == 0), "conv3x3_small: upsampled size must be even");
-    EDS_REQUIRE((((uintptr_t)x | (uintptr_t)w | (uintptr_t)y) & 15) == 0 && (((uintptr_t)bias | (uintptr_t)cgate) & 15) == 0,
+    EDS_REQUIRE((((uintptr_t)x | (uintptr_t)w | (uintptr_t)y) & 15) == 0 && ((uintptr_t)bias & 15) == 0,
                 "conv3x3_small: pointers must be 16-byte aligned");
     cudaStream_t s = as_stream(stream);
-#define EDS_SMALL_CASE(CI, CO)                                                                                         \
-    if (C == CI && Cout == CO) {                                                                                       \
-        if (up_mode == EDS_UP_NONE) return small_launch<CI, CO, 0>(x, cgate, sgate, N, H, W, w, bias, relu, y, s);     \
-        if (up_mode == EDS_UP_NEAREST) return small_launch<CI, CO, 1>(x, cgate, sgate, N, H, W, w, bias, relu, y, s);  \
-        return small_launch<CI, CO, 2>(x, cgate, sgate, N, H, W, w, bias, relu, y, s);                                 \
-    }
-    EDS_SMALL_CASE(32, 16) EDS_SMALL_CASE(16, 16) EDS_SMALL_CASE(32, 32) EDS_SMALL_CASE(16, 32)
-#undef EDS_SMALL_CASE
-    set_error("conv3x3_small: unreachable");
-    return EDS_ERR_INVALID;
+    if (Cout == 16) return small_launch<16>(x, N, H, W, w, bias, relu, y, s);
+    return small_launch<32>(x, N, H, W, w, bias, relu, y, s);
 }

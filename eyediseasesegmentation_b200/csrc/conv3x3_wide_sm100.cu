@@ -36,7 +36,6 @@
 // its 24 MMAs instead of by the weight re-load.
 #include "tc_ptx.cuh"
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -334,10 +333,6 @@ static int wide_launch(const void* x, int C0, const void* x1, int C1, int N, int
     p.y = (__nv_bfloat16*)y;
     p.C = C;
     p.block_k = ((C0 | C1) % 64 == 0) ? 64 : ((C0 | C1) % 32 == 0 ? 32 : 16);   // divides both inputs
-    if (const char* bk = getenv("EDS_WIDE_BK")) {          // developer switch: finer pipeline stages
-        const int v = atoi(bk);
-        if ((v == 32 || v == 16) && (C0 | C1) % v == 0) p.block_k = std::min(p.block_k, v);
-    }
     p.k_chunks = C / p.block_k;
     p.k_split = C0 / p.block_k;
     p.bn = Cout;
@@ -360,8 +355,7 @@ static int wide_launch(const void* x, int C0, const void* x1, int C1, int N, int
     const int barrier_bytes = 128 + 64 * 4;   // 13 barriers + TMEM slot in the first 128 B, then the bias
     const int budget = 227 * 1024 - 1024 - barrier_bytes;
     const int b_all = p.k_chunks * 9 * p.b_box_bytes;               // the whole weight tensor
-    static const bool no_resident = getenv("EDS_WIDE_RESIDENT") && atoi(getenv("EDS_WIDE_RESIDENT")) == 0;
-    p.b_resident = !no_resident && b_all + 3 * p.a_slab_bytes <= budget;
+    p.b_resident = b_all + 3 * p.a_slab_bytes <= budget;
     p.b_region_bytes = p.b_resident ? ((b_all + 1023) & ~1023) : 0;
     // the 9 boxes of a chunk are contiguous: the 3 of a kernel row stack into one [3 * bn][block_k] operand
     p.stage_bytes = p.b_resident ? p.a_slab_bytes : ((p.a_slab_bytes + 9 * p.b_box_bytes + 1023) & ~1023);
@@ -373,10 +367,9 @@ static int wide_launch(const void* x, int C0, const void* x1, int C1, int N, int
     // staged epilogue when 8 x 4 KB fit behind the ring (the resident-weight 64 -> 64 layers; the multi-chunk layers
     // hide their epilogue behind the MMAs of the next tile and need the room for the second stage).
     // layout: [weights][ring][barriers + bias (barrier_bytes)][pad to 1024][staging]
-    static const bool no_staging = getenv("EDS_WIDE_STAGED") && atoi(getenv("EDS_WIDE_STAGED")) == 0;
     const int after_bars = p.b_region_bytes + p.stages * p.stage_bytes + barrier_bytes;
     p.staging_off = (after_bars + 1023) & ~1023;
-    p.staged = !no_staging && p.bn == 64 && p.block_k == 64 && p.staging_off + 8 * 4096 + 1024 <= 227 * 1024;
+    p.staged = p.bn == 64 && p.block_k == 64 && p.staging_off + 8 * 4096 + 1024 <= 227 * 1024;
     const size_t smem = (p.staged ? (size_t)p.staging_off + 8 * 4096 : (size_t)after_bars) + 1024;
     EDS_REQUIRE(smem <= 227 * 1024 && p.tmem_cols <= 512, "conv3x3_wide: tile does not fit (smem %zu, tmem %d)", smem,
                 p.tmem_cols);

@@ -27,7 +27,6 @@
 #include "tc_ptx.cuh"
 #include <algorithm>
 #include <climits>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -52,9 +51,8 @@ struct IgemmParams {
     int tw_log2, th_log2, TW, TH, TN;
     int tiles_w, tiles_h;
     int N, Ho, Wo, Cout, relu;
-    int total_tiles;
     CUtensorMap y_map;      // output [Cout][Wo][Ho][N], box [st_ch][TW][TH][TN]
-    int debug;              // developer timing switches (EDS_IGEMM_DEBUG): 1 = no bulk store, 2 = empty epilogue
+    int total_tiles;        // after y_map: nvcc 12.9 then spills 76 / 96 B (stores / loads) instead of 84 / 112 B
     int st_ch, st_bytes, st_bufs, st_mode;   // epilogue staging: channels per TMA store, bytes per buffer, buffers per half, swizzle mode
     int stages, a_stage_bytes, b_stage_bytes, tmem_cols;
     uint32_t idesc;
@@ -245,7 +243,7 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
             mbar_wait(&tmem_full_bar[buf], (uint32_t)((t >> 1) & 1));
             tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * p.block_n);
-            for (int grp = half; grp < n_groups && !(p.debug & 2); grp += 2) {
+            for (int grp = half; grp < n_groups; grp += 2) {
                 uint8_t* sdst = my_stage + (size_t)sbuf * p.st_bytes;
                 // all TMEM loads of the group are issued before the single wait
                 uint32_t r[4][16];
@@ -265,8 +263,7 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                                        : make_float4(0.f, 0.f, 0.f, 0.f);
                 // the store that last read this staging buffer must have finished reading it
                 if (issuer) {
-                    if (p.st_bufs == 4) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(3) : "memory");
-                    else if (p.st_bufs == 2) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(1) : "memory");
+                    if (p.st_bufs == 2) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(1) : "memory");
                     else asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(0) : "memory");
                 }
                 asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");
@@ -335,7 +332,7 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                 }
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");
-                if (issuer && !(p.debug & 1)) {
+                if (issuer) {
                     asm volatile(
                         "cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
                         ::"l"(&p.y_map), "r"(smem_u32(sdst)), "r"(co0 + grp * p.st_ch), "r"(w0), "r"(h0), "r"(n0)
@@ -366,7 +363,6 @@ static EncodeTiledFn g_encode = nullptr;
 static std::once_flag g_igemm_once;
 static int g_igemm_init_rc = EDS_OK;
 static int g_num_sms = 148;
-static CUtensorMapL2promotion g_l2_promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
 
 static void igemm_init_once() {
     void* fn = nullptr;
@@ -379,11 +375,6 @@ static void igemm_init_once() {
         return;
     }
     g_encode = reinterpret_cast<EncodeTiledFn>(fn);
-    if (const char* pr = getenv("EDS_L2_PROMO")) {
-        const int v = atoi(pr);
-        g_l2_promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                     : v == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-    }
 }
 
 static PerDevice g_igemm_attr_once;       // the shared-memory opt-in belongs to a device's context
@@ -415,7 +406,7 @@ int tmap_encode_bf16(CUtensorMap* map, const void* base, int rank, const cuuint6
                      const cuuint32_t* box, CUtensorMapSwizzle swz, const char* what) {
     cuuint32_t ones[5] = {1, 1, 1, 1, 1};
     CUresult r = g_encode(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims,
-                          strides, box, ones, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, g_l2_promo,
+                          strides, box, ones, CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
         set_error("conv_igemm: cuTensorMapEncodeTiled(%s) failed with CUresult %d", what, (int)r);
@@ -477,7 +468,6 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     p.block_n = bn;
     p.n_tiles = Cout / bn;
     p.N = N; p.Ho = Ho; p.Wo = Wo; p.Cout = Cout; p.relu = relu;
-    if (const char* dbg = getenv("EDS_IGEMM_DEBUG")) p.debug = atoi(dbg);
 
     // pixel tile TN x TH x TW = 128 minimising the number of tiles (ties -> wider rows)
     int best_tiles = INT32_MAX, best_tw = 8;
@@ -513,11 +503,6 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     p.st_bytes = kTileM * p.st_ch * 2;                                 // 16 / 8 / 4 KB
     // short reductions are store-bound: overlap the bulk stores with the next groups (st_bufs per half in flight)
     p.st_bufs = k_iters <= 8 ? 2 : 1;
-    {
-        static const int force = getenv("EDS_IGEMM_STBUFS") ? atoi(getenv("EDS_IGEMM_STBUFS")) : 0;
-        const int short_bufs = force ? force : 2;
-        if (k_iters <= 4 && (short_bufs == 1 || short_bufs == 2 || short_bufs == 4)) p.st_bufs = short_bufs;
-    }
     // one persistent CTA per SM: the rest of the shared memory is one TMA ring
     const int res_bytes = residual ? 4 * p.st_bytes : 0;               // two residual buffers per epilogue half
     // one persistent CTA per SM: the rest of the shared memory is one TMA ring of at least two stages (fewer staging

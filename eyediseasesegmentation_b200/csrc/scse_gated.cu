@@ -20,7 +20,6 @@
 // Traffic per decoder block: 2 reads of the sources + 1 write of the concat (was 1 read of the sources,
 // 2 writes + 1 read of the concat, and 2 reads + 1 write of the block output for attention2).
 #include "common.cuh"
-#include <cstdlib>
 #include <cstring>
 
 namespace eds {
@@ -349,92 +348,75 @@ __device__ __forceinline__ void ld_gated(const T* p, const float2 (&cg)[4], cons
     }
 }
 
+// ---- pass A, upsampled part: the channels of source 0 ----------------------------------------------------------------
 // One thread = one 8-channel vector of a 2 x 4 OUTPUT block = two adjacent low-res pixels (i, 2jj),
 // (i, 2jj+1) of source 0 and their 3 x 4 neighbourhood (12 loads feed 8 outputs; the vertical lerps of
-// the two inner columns are shared), or the 8 same-resolution pixels of a skip source.  Index arithmetic
-// and bf16 unpacking were most of the instructions of the 2 x 2 version; the wider block halves them
-// per output.  grid.x = N*h rows of blocks, grid.y covers (jj, vector) of a row; consecutive threads own
-// consecutive vectors of the same block, so every global access of a warp is a contiguous run.  All
-// lerps / gates run on the packed fp32 pipe.
-// PART 0 writes the channels of the upsampled source 0 (register-heavy: 12 vectors in flight), PART 1 the
-// channels of the same-resolution sources (a light streaming kernel).
-template <typename T, int PART>
+// the two inner columns are shared).  Index arithmetic and bf16 unpacking were most of the instructions
+// of the 2 x 2 version; the wider block halves them per output.  grid.x = N*h rows of blocks, grid.y
+// covers (jj, vector) of a row; consecutive threads own consecutive vectors of the same block, so every
+// global access of a warp is a contiguous run.  All lerps / gates run on the packed fp32 pipe.
+template <typename T>
 __global__ void __launch_bounds__(256, 2)
 concat_gated_kernel(CatSrcs src, int h, int w, int mode, int Ctot, const float* __restrict__ cgate1,
                     const float* __restrict__ sgate1, T* __restrict__ y, int y_stride, int y_coff) {
-    const uint32_t C8a = (uint32_t)src.s[0].C / 8;
-    const uint32_t C8 = PART == 0 ? C8a : (uint32_t)Ctot / 8 - C8a;     // vectors per pixel of this part
+    const GatedSrc s = src.s[0];
+    const uint32_t C8 = (uint32_t)s.C / 8;                              // vectors per pixel of source 0
     const uint32_t wp = (uint32_t)(w + 1) / 2;                          // column pairs per low-res row
     const uint32_t col = blockIdx.y * blockDim.x + threadIdx.x;
     if (col >= wp * C8) return;
     const int jj = (int)(col / C8);
-    const int c8 = (int)(col - (uint32_t)jj * C8) + (PART == 0 ? 0 : (int)C8a);
+    const int c8 = (int)(col - (uint32_t)jj * C8);
     const int n = (int)(blockIdx.x / (uint32_t)h);
     const int i = (int)(blockIdx.x - (uint32_t)n * h);
     const int j0 = 2 * jj;
     const bool second = j0 + 1 < w;                 // odd widths: the last pair has one column
     const int H = 2 * h, W = 2 * w;
-    int c = c8 * 8, k = 0;
-    if (PART == 1)
-        while (k < src.n - 1 && c >= src.s[k].C) { c -= src.s[k].C; ++k; }
-    const GatedSrc s = src.s[k];
+    const int c = c8 * 8;
     const bool gated = s.cgate != nullptr;
     float2 cg[4];
     if (gated) ld8f(s.cgate + (int64_t)n * s.C + c, cg);
     float2 o[8][4];                                 // [row * 4 + column of the block][channel pair]
-    if (PART == 0) {
-        const T* xp = reinterpret_cast<const T*>(s.x) + (int64_t)n * h * w * s.C + c;
-        const float* sg = s.sgate + (int64_t)n * h * w;      // only dereferenced when gated
-        if (mode == EDS_UP_NEAREST) {
-            const int p0 = i * w + j0, p1 = i * w + min(j0 + 1, w - 1);
-            ld_gated<T>(xp + (int64_t)p0 * s.C, cg, sg + p0, gated, o[0]);
-            ld_gated<T>(xp + (int64_t)p1 * s.C, cg, sg + p1, gated, o[2]);
+    const T* xp = reinterpret_cast<const T*>(s.x) + (int64_t)n * h * w * s.C + c;
+    const float* sg = s.sgate + (int64_t)n * h * w;      // only dereferenced when gated
+    if (mode == EDS_UP_NEAREST) {
+        const int p0 = i * w + j0, p1 = i * w + min(j0 + 1, w - 1);
+        ld_gated<T>(xp + (int64_t)p0 * s.C, cg, sg + p0, gated, o[0]);
+        ld_gated<T>(xp + (int64_t)p1 * s.C, cg, sg + p1, gated, o[2]);
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                o[1][q] = o[4][q] = o[5][q] = o[0][q];
-                o[3][q] = o[6][q] = o[7][q] = o[2][q];
-            }
-        } else {
-            const int r[3] = {max(i - 1, 0) * w, i * w, min(i + 1, h - 1) * w};
-            const int cc[4] = {max(j0 - 1, 0), j0, min(j0 + 1, w - 1), min(j0 + 2, w - 1)};
-            float2 top[4][4], bot[4][4];
-            const float2 q25 = f2(0.25f), q75 = f2(0.75f);
-#pragma unroll
-            for (int a = 0; a < 4; ++a) {
-                float2 v0[4], v1[4], v2[4];
-                ld_gated<T>(xp + (int64_t)(r[0] + cc[a]) * s.C, cg, sg + r[0] + cc[a], gated, v0);
-                ld_gated<T>(xp + (int64_t)(r[1] + cc[a]) * s.C, cg, sg + r[1] + cc[a], gated, v1);
-                ld_gated<T>(xp + (int64_t)(r[2] + cc[a]) * s.C, cg, sg + r[2] + cc[a], gated, v2);
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const float2 m = __fmul2_rn(q75, v1[q]);
-                    top[a][q] = __ffma2_rn(q25, v0[q], m);
-                    bot[a][q] = __ffma2_rn(q25, v2[q], m);
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const float2 t1 = __fmul2_rn(q75, top[1][q]), t2 = __fmul2_rn(q75, top[2][q]);
-                const float2 b1 = __fmul2_rn(q75, bot[1][q]), b2 = __fmul2_rn(q75, bot[2][q]);
-                o[0][q] = __ffma2_rn(q25, top[0][q], t1);
-                o[1][q] = __ffma2_rn(q25, top[2][q], t1);
-                o[2][q] = __ffma2_rn(q25, top[1][q], t2);
-                o[3][q] = __ffma2_rn(q25, top[3][q], t2);
-                o[4][q] = __ffma2_rn(q25, bot[0][q], b1);
-                o[5][q] = __ffma2_rn(q25, bot[2][q], b1);
-                o[6][q] = __ffma2_rn(q25, bot[1][q], b2);
-                o[7][q] = __ffma2_rn(q25, bot[3][q], b2);
-            }
+        for (int q = 0; q < 4; ++q) {
+            o[1][q] = o[4][q] = o[5][q] = o[0][q];
+            o[3][q] = o[6][q] = o[7][q] = o[2][q];
         }
     } else {
-        const T* xp = reinterpret_cast<const T*>(s.x) + (int64_t)n * H * W * s.C + c;
-        const float* sg = s.sgate + (int64_t)n * H * W;
+        const int r[3] = {max(i - 1, 0) * w, i * w, min(i + 1, h - 1) * w};
+        const int cc[4] = {max(j0 - 1, 0), j0, min(j0 + 1, w - 1), min(j0 + 2, w - 1)};
+        float2 top[4][4], bot[4][4];
+        const float2 q25 = f2(0.25f), q75 = f2(0.75f);
 #pragma unroll
-        for (int d = 0; d < 8; ++d) {
-            // columns 2, 3 of the block do not exist for the last pair of an odd width: clamp the address
-            const int px = min(2 * j0 + (d & 3), W - 1);
-            const int p = (2 * i + (d >> 2)) * W + px;
-            ld_gated<T>(xp + (int64_t)p * s.C, cg, sg + p, gated, o[d]);
+        for (int a = 0; a < 4; ++a) {
+            float2 v0[4], v1[4], v2[4];
+            ld_gated<T>(xp + (int64_t)(r[0] + cc[a]) * s.C, cg, sg + r[0] + cc[a], gated, v0);
+            ld_gated<T>(xp + (int64_t)(r[1] + cc[a]) * s.C, cg, sg + r[1] + cc[a], gated, v1);
+            ld_gated<T>(xp + (int64_t)(r[2] + cc[a]) * s.C, cg, sg + r[2] + cc[a], gated, v2);
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const float2 m = __fmul2_rn(q75, v1[q]);
+                top[a][q] = __ffma2_rn(q25, v0[q], m);
+                bot[a][q] = __ffma2_rn(q25, v2[q], m);
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const float2 t1 = __fmul2_rn(q75, top[1][q]), t2 = __fmul2_rn(q75, top[2][q]);
+            const float2 b1 = __fmul2_rn(q75, bot[1][q]), b2 = __fmul2_rn(q75, bot[2][q]);
+            o[0][q] = __ffma2_rn(q25, top[0][q], t1);
+            o[1][q] = __ffma2_rn(q25, top[2][q], t1);
+            o[2][q] = __ffma2_rn(q25, top[1][q], t2);
+            o[3][q] = __ffma2_rn(q25, top[3][q], t2);
+            o[4][q] = __ffma2_rn(q25, bot[0][q], b1);
+            o[5][q] = __ffma2_rn(q25, bot[2][q], b1);
+            o[6][q] = __ffma2_rn(q25, bot[1][q], b2);
+            o[7][q] = __ffma2_rn(q25, bot[3][q], b2);
         }
     }
     const int64_t p00 = ((int64_t)n * H + 2 * i) * W + 2 * j0;     // output pixel (2i, 2 j0)
@@ -477,10 +459,9 @@ concat_gated_kernel(CatSrcs src, int h, int w, int mode, int Ctot, const float* 
 }
 
 // ---- pass B, same-resolution (skip) part: a lean streaming kernel ---------------------------------------------------
-// concat_gated_kernel<T, 1> keeps eight output vectors per thread (128 registers, spills in the bf16 build, two CTAs
-// per SM, ncu: 23 % occupancy and neither DRAM nor issue saturated -- latency-bound).  One thread here = one 8-channel
-// vector of FOUR consecutive pixels of a row: half the registers, twice the resident threads, the same arithmetic in
-// the same order (bit-identical results).  grid.x = N * H rows, grid.y covers (quad, vector) of a row.
+// One thread = one 8-channel vector of FOUR consecutive pixels of a row.  (A version that kept eight output vectors
+// per thread, the 2 x 4 block of pass A, needed 128 registers, spilled in the bf16 build and was latency-bound at
+// 23 % occupancy.)  grid.x = N * H rows, grid.y covers (quad, vector) of a row.
 template <typename T>
 __global__ void __launch_bounds__(256, 3)
 concat_skip_kernel(CatSrcs src, int H, int W, int Ctot, const float* __restrict__ cgate1,
@@ -694,8 +675,10 @@ static int concat_gated_launch(const eds_gated_src* srcs, int n_srcs, int N, int
             cs.s[k].x = nullptr; cs.s[k].cgate = nullptr; cs.s[k].sgate = nullptr; cs.s[k].C = 0;
         }
     }
-    EDS_REQUIRE((int64_t)w * (Ctot / 8) < (1ll << 24) && (int64_t)N * h < (1ll << 31), "concat_gated: map too large");
     const int c8a = cs.s[0].C / 8, c8b = Ctot / 8 - c8a;
+    EDS_REQUIRE((int64_t)w * (Ctot / 8) < (1ll << 24) && (int64_t)N * h < (1ll << 31), "concat_gated: map too large");
+    EDS_REQUIRE(c8b == 0 || (int64_t)N * 2 * h < (1ll << 31), "concat_gated: map too large (N * 2h = %lld rows)",
+                (long long)N * 2 * h);
     const int wp = (w + 1) / 2;
     EDS_REQUIRE(!y_skip || c8b > 0, "concat_gated: y_skip given without skip sources");
     // one destination of Ctot channels, or two dense ones (upsampled part / skip part)
@@ -704,22 +687,15 @@ static int concat_gated_launch(const eds_gated_src* srcs, int n_srcs, int N, int
     // per thread -- measured 2.4-2.5 TB/s against 3.3-3.7 TB/s for the per-thread kernel on the benchmark's layers,
     // scripts/dev_concat_probe.py: one barrier per small tile and 104 registers leave too little in flight.)
     dim3 grid_a((unsigned)(N * h), (unsigned)ceil_div(wp * c8a, 256));
-    EDS_DISPATCH_DTYPE(dtype, T, (concat_gated_kernel<T, 0><<<grid_a, 256, 0, as_stream(stream)>>>(
+    EDS_DISPATCH_DTYPE(dtype, T, (concat_gated_kernel<T><<<grid_a, 256, 0, as_stream(stream)>>>(
                                      cs, h, w, mode, Ctot, cgate, sgate, (T*)y, stride_a, 0)));
     if (c8b > 0) {
         void* yb = y_skip ? y_skip : y;
         const int stride_b = y_skip ? Ctot - cs.s[0].C : Ctot;
         const int coff_b = y_skip ? cs.s[0].C : 0;
-        static const bool lean_off = getenv("EDS_CONCAT_SKIP_LEAN") && atoi(getenv("EDS_CONCAT_SKIP_LEAN")) == 0;
-        if (!lean_off && (int64_t)N * 2 * h < (1ll << 31)) {
-            dim3 grid_s((unsigned)(N * 2 * h), (unsigned)ceil_div(ceil_div(2 * w, 4) * c8b, 256));
-            EDS_DISPATCH_DTYPE(dtype, T, (concat_skip_kernel<T><<<grid_s, 256, 0, as_stream(stream)>>>(
-                                             cs, 2 * h, 2 * w, Ctot, cgate, sgate, (T*)yb, stride_b, coff_b)));
-        } else {
-            dim3 grid_b((unsigned)(N * h), (unsigned)ceil_div(wp * c8b, 256));
-            EDS_DISPATCH_DTYPE(dtype, T, (concat_gated_kernel<T, 1><<<grid_b, 256, 0, as_stream(stream)>>>(
-                                             cs, h, w, mode, Ctot, cgate, sgate, (T*)yb, stride_b, coff_b)));
-        }
+        dim3 grid_s((unsigned)(N * 2 * h), (unsigned)ceil_div(ceil_div(2 * w, 4) * c8b, 256));
+        EDS_DISPATCH_DTYPE(dtype, T, (concat_skip_kernel<T><<<grid_s, 256, 0, as_stream(stream)>>>(
+                                         cs, 2 * h, 2 * w, Ctot, cgate, sgate, (T*)yb, stride_b, coff_b)));
     }
     return check_launch("concat_gated_kernel");
 }

@@ -2,15 +2,16 @@
 // BatchNorm + ReLU, TTA views folded into the loader (same contract as stem.cu, which keeps the fp32
 // parity mode).
 //
-// GEMM view per CTA: D[128 pixels][64 couts] = A[128][K] . B[64][K]^T with K ordered (c, r, s') where the
+// GEMM view per CTA: D[256 pixels][64 couts] = A[256][K] . B[64][K]^T with K ordered (c, r, s') where the
 // 7 horizontal taps are padded to s' = 0..7 (weight 0 for s' = 7): K = 3 * 7 * 8 = 168 (+8 zero) = 176.
-// With that order the im2col row of a pixel is, per (c, r), EIGHT CONSECUTIVE input pixels of one patch
-// row, so building A in shared memory is one 16-byte copy per (pixel, c, r) -- 21 copies per pixel instead
-// of 147 scalar gathers.  8 warps x (16 pixels x 64 couts) x 11 k-steps of mma.sync.m16n8k16 (bf16 in, fp32
-// accumulate).  Cin = 3 rules out a TMA / tcgen05 formulation (there is no dense channel axis to tile);
-// the stem is 0.3 % of the network's FLOPs and was 4 % of its time on the packed fp32 pipe.
+// With that order the two bf16 of an A fragment a lane needs are the patch pixels [c][2 py + r][2 px + 2t, + 1],
+// one aligned 32-bit word, so A is read straight from the bf16 input patch and no im2col matrix is built.
+// 8 warps x (2 output rows x 16 pixels x 64 couts) x 11 k-steps of mma.sync.m16n8k16 (bf16 in, fp32 accumulate):
+// a warp owns two output rows so one B fragment read from shared memory feeds two MMAs, and the 16 x 16-pixel
+// tile copies the 23.5 KB weight tile once per 256 pixels.  Cin = 3 rules out a TMA / tcgen05 formulation (there
+// is no dense channel axis to tile); the stem is 0.3 % of the network's FLOPs and was 4 % of its time on the
+// packed fp32 pipe.
 #include "common.cuh"
-#include <cstdlib>
 
 namespace eds {
 
@@ -18,13 +19,9 @@ struct StemViews {
     int m[8][6];
 };
 
-constexpr int kSmTileH = 8, kSmTileW = 16;                 // output pixels per CTA: 8 rows x 16 cols
-constexpr int kSmPatchH = 2 * kSmTileH + 5;                // 21 input rows
-constexpr int kSmPatchW = 40;                              // 2*16+5 = 37 input cols (+3 pad)
 constexpr int kSmGroups = 22;                              // 21 (c, r) groups of 8 taps + 1 zero group
 constexpr int kSmK = kSmGroups * 8;                        // 176
-constexpr int kSmPitch = 184;                              // bf16 per A / B row (conflict-free fragments)
-constexpr size_t kSmSmemBytes = (size_t)(3 * kSmPatchH * kSmPatchW + 128 * kSmPitch + 64 * kSmPitch) * 2;
+constexpr int kSmPitch = 184;                              // bf16 per B row (conflict-free fragments)
 
 __device__ __forceinline__ void stem_mma_16816(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3,
                                                uint32_t b0, uint32_t b1) {
@@ -34,111 +31,6 @@ __device__ __forceinline__ void stem_mma_16816(float (&c)[4], uint32_t a0, uint3
         : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-__global__ void __launch_bounds__(256)
-stem_conv_mma_kernel(const float* __restrict__ x, int B, int H, int W, StemViews views,
-                     const __nv_bfloat16* __restrict__ w_packed, const float* __restrict__ bias,
-                     __nv_bfloat16* __restrict__ y) {
-    extern __shared__ __align__(16) uint8_t sm_raw[];
-    __nv_bfloat16* s_in = reinterpret_cast<__nv_bfloat16*>(sm_raw);                 // [3][21][40]
-    __nv_bfloat16* s_a = s_in + 3 * kSmPatchH * kSmPatchW;                          // [128][184]
-    __nv_bfloat16* s_b = s_a + 128 * kSmPitch;                                      // [64][184]
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int Ho = H / 2, Wo = W / 2;
-    const int img = blockIdx.z;         // v * B + b
-    const int v = img / B, b = img % B;
-    const int oy0 = blockIdx.y * kSmTileH, ox0 = blockIdx.x * kSmTileW;
-    const __nv_bfloat16 zero = __float2bfloat16_rn(0.f);
-
-    // packed weights B[cout][184] (eds_stem_pack_weights): a straight 23.5 KB copy
-    for (int i = tid; i < 64 * kSmPitch / 8; i += 256)
-        reinterpret_cast<uint4*>(s_b)[i] = __ldg(reinterpret_cast<const uint4*>(w_packed) + i);
-    // input patch of the augmented view, bf16
-    const int* m = views.m[v];
-    const float* xb = x + (int64_t)b * 3 * H * W;
-    for (int i = tid; i < 3 * kSmPatchH * kSmPatchW; i += 256) {
-        const int c = i / (kSmPatchH * kSmPatchW);
-        const int rem = i - c * (kSmPatchH * kSmPatchW);
-        const int py = rem / kSmPatchW, px = rem - py * kSmPatchW;
-        const int iy = 2 * oy0 - 3 + py, ix = 2 * ox0 - 3 + px;  // coordinates in the augmented view
-        float val = 0.f;
-        if (iy >= 0 && iy < H && ix >= 0 && ix < W) {
-            const int sy = m[0] * iy + m[1] * ix + m[2];
-            const int sx = m[3] * iy + m[4] * ix + m[5];
-            val = __ldg(xb + ((int64_t)c * H + sy) * W + sx);
-        }
-        s_in[i] = __float2bfloat16_rn(val);
-    }
-    __syncthreads();
-    // im2col: A[p][gq*8 .. +7] = patch[c][2*py + r][2*px .. 2*px + 7]   (one 16-byte store per (p, gq))
-    for (int i = tid; i < 128 * kSmGroups; i += 256) {
-        const int p = i / kSmGroups, gq = i - p * kSmGroups;
-        uint4 val = make_uint4(0, 0, 0, 0);
-        if (gq < 21) {
-            const int c = gq / 7, r = gq - c * 7;
-            const int py = p >> 4, px = p & 15;
-            const uint32_t* src = reinterpret_cast<const uint32_t*>(s_in + (c * kSmPatchH + 2 * py + r) * kSmPatchW + 2 * px);
-            val = make_uint4(src[0], src[1], src[2], src[3]);
-        }
-        *reinterpret_cast<uint4*>(s_a + p * kSmPitch + gq * 8) = val;
-    }
-    __syncthreads();
-
-    // warp w: output row w of the tile (16 pixels) x 64 couts
-    const int g = lane >> 2, t = lane & 3;
-    float acc[8][4];
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) acc[nt][i] = 0.f;
-    const __nv_bfloat16* a_lo = s_a + (warp * 16 + g) * kSmPitch + 2 * t;
-    const __nv_bfloat16* a_hi = a_lo + 8 * kSmPitch;
-#pragma unroll
-    for (int ks = 0; ks < kSmK / 16; ++ks) {
-        const uint32_t a0 = *reinterpret_cast<const uint32_t*>(a_lo + ks * 16);
-        const uint32_t a1 = *reinterpret_cast<const uint32_t*>(a_hi + ks * 16);
-        const uint32_t a2 = *reinterpret_cast<const uint32_t*>(a_lo + ks * 16 + 8);
-        const uint32_t a3 = *reinterpret_cast<const uint32_t*>(a_hi + ks * 16 + 8);
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-            const __nv_bfloat16* bp = s_b + (nt * 8 + g) * kSmPitch + ks * 16 + 2 * t;
-            stem_mma_16816(acc[nt], a0, a1, a2, a3, *reinterpret_cast<const uint32_t*>(bp),
-                           *reinterpret_cast<const uint32_t*>(bp + 8));
-        }
-    }
-    // bias + ReLU + bf16 -> staging tile [128][72] in the (now free) A region -> 16-byte coalesced stores
-    __syncthreads();
-    __nv_bfloat16* s_out = s_a;
-    constexpr int kOutPitch = 72;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-        const float2 bb = *reinterpret_cast<const float2*>(bias + nt * 8 + 2 * t);
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-            const float v0 = fmaxf(acc[nt][2 * half] + bb.x, 0.f), v1 = fmaxf(acc[nt][2 * half + 1] + bb.y, 0.f);
-            *reinterpret_cast<__nv_bfloat162*>(s_out + (warp * 16 + g + half * 8) * kOutPitch + nt * 8 + 2 * t) =
-                __floats2bfloat162_rn(v0, v1);
-        }
-    }
-    __syncthreads();
-    for (int i = tid; i < 128 * 8; i += 256) {
-        const int p = i >> 3, ch8 = i & 7;
-        const int oy = oy0 + (p >> 4), ox = ox0 + (p & 15);
-        if (oy < Ho && ox < Wo)
-            *reinterpret_cast<uint4*>(y + (((int64_t)img * Ho + oy) * Wo + ox) * 64 + ch8 * 8) =
-                *reinterpret_cast<const uint4*>(s_out + p * kOutPitch + ch8 * 8);
-    }
-}
-
-// ---- round 2: no im2col copy, two output rows per warp ---------------------------------------------------------
-// ncu on the kernel above (profiles/r02_small_kernels_full.md #0): 57 % of the shared-memory wavefront budget,
-// tensor pipe 21 % active, 0.16 of the HBM write roof -- it is bound by shared-memory BYTES: every warp re-reads the
-// whole 22.5 KB weight tile for its 16 pixels and the patch is copied once more into an explicit A matrix.  Here
-//   * the A fragments are read straight from the patch: with K ordered (c, r, s') the two bf16 a lane needs are the
-//     patch pixels [c][2 py + r][2 px + 2t, + 1], one aligned 32-bit word (lanes with equal g + t share a word);
-//   * a warp owns TWO output rows (two m16 tiles), so a B fragment read from shared memory feeds two MMAs;
-//   * the tile is 16 x 16 output pixels: the weight tile is copied once per 256 pixels instead of once per 128.
-// Shared memory traffic per output pixel drops from ~2.7 KB to ~1.5 KB; same K order, same products, same fp32
-// accumulation order per output as the kernel above (bit-identical results).
 constexpr int kS2TileH = 16, kS2TileW = 16;
 constexpr int kS2PatchH = 2 * kS2TileH + 5;                // 37 input rows
 constexpr int kS2PatchW = 40;                              // 37 input cols (+3: tap s' = 7 of the last pixel reads col 37)
@@ -260,17 +152,8 @@ int stem_conv_mma_launch(const float* x, int B, int H, int W, int V, const int* 
     StemViews views;
     for (int v = 0; v < V; ++v)
         for (int q = 0; q < 6; ++q) views.m[v][q] = maps[v * 6 + q];
-    static const bool v1 = getenv("EDS_STEM_V1") && atoi(getenv("EDS_STEM_V1")) == 1;     // A/B switch: the round-1 kernel
-    if (v1) {
-        static PerDevice once;
-        if (int rc = smem_opt_in(once, stem_conv_mma_kernel, (int)kSmSmemBytes, "stem_conv_mma")) return rc;
-        dim3 grid(ceil_div(W / 2, kSmTileW), ceil_div(H / 2, kSmTileH), B * V);
-        stem_conv_mma_kernel<<<grid, 256, kSmSmemBytes, stream>>>(x, B, H, W, views, (const __nv_bfloat16*)w_packed,
-                                                                bias, (__nv_bfloat16*)y);
-        return check_launch("stem_conv_mma_kernel");
-    }
-    static PerDevice once16;
-    if (int rc = smem_opt_in(once16, stem_conv_mma16_kernel, (int)kS2SmemBytes, "stem_conv_mma16")) return rc;
+    static PerDevice once;
+    if (int rc = smem_opt_in(once, stem_conv_mma16_kernel, (int)kS2SmemBytes, "stem_conv_mma16")) return rc;
     dim3 grid(ceil_div(W / 2, kS2TileW), ceil_div(H / 2, kS2TileH), B * V);
     stem_conv_mma16_kernel<<<grid, 256, kS2SmemBytes, stream>>>(x, B, H, W, views, (const __nv_bfloat16*)w_packed, bias,
                                                               (__nv_bfloat16*)y);

@@ -12,7 +12,6 @@
 // pieces (generic TTA wrapper, ensemble mean, whole-image path, other tile sizes); the Gaussian kernels are an
 // opt-in blend mode with no reference counterpart.
 #include "common.cuh"
-#include <cstdlib>
 
 namespace eds {
 
@@ -660,8 +659,7 @@ extern "C" int eds_tta_merge(const float* logits, int V, int B, int S, const int
     if (int rc = check_view_maps(view_maps_host, V, S, &maps, "tta_merge")) return rc;
     // 64x64 vector kernel when the tile size and every column offset keep the 16-byte loads aligned
     const bool vec = merge_vector_ok(maps, V, S, logits, prob);
-    static const bool force_scalar = getenv("EDS_MERGE_SCALAR") && atoi(getenv("EDS_MERGE_SCALAR")) != 0;
-    if (vec && !force_scalar) {
+    if (vec) {
         const int smem = 4 * kMergeTile * kMergeTile * (int)sizeof(float);
         // 512 threads x 2 rows measured best on B200 (50.0 us for 48 maps of 1024^2; 256 x 4 rows: 53.2 us;
         // 3 CTAs/SM at 80 registers spills: 59.4 us)

@@ -19,19 +19,11 @@ LAUNCHES = [0]
 #: when set to a list, conv2d(impl="tc") appends (algorithmic_flops, start_event, end_event)
 CONV_TRACE = None
 #: 3x3 s1 p1 convolutions with Cout <= 128 on maps at least this large take the halo-reuse kernel
-#: (0 disables it; EDS_HALO_MIN_HW overrides)
-HALO_MIN_HW = int(__import__("os").environ.get("EDS_HALO_MIN_HW", "64"))
+HALO_MIN_HW = 64
 #: 3x3 layers with Cout <= 64 run on the dw-grouped wide-N kernel (conv3x3_wide_sm100.cu) when the map is at
-#: least WIDE_MIN_HW on its short side and the reduction has at least WIDE_MIN_CIN channels (EDS_WIDE_CONV=0 off)
-WIDE_CONV = __import__("os").environ.get("EDS_WIDE_CONV", "1") != "0"
-WIDE_MIN_HW = int(__import__("os").environ.get("EDS_WIDE_MIN_HW", "64"))
-WIDE_MIN_CIN = int(__import__("os").environ.get("EDS_WIDE_MIN_CIN", "16"))
-#: 3x3 s1 p1 convolutions with C and Cout in {16, 32} (the full-resolution decoder tail) take the mma.sync
-#: kernel of conv3x3_small.cu (EDS_SMALL_CONV=0 sends them to the implicit-GEMM kernels)
-SMALL_CONV = __import__("os").environ.get("EDS_SMALL_CONV", "1") != "0"
-#: fuse the x2 upsampling of the last decoder block into conv1's tile loader (conv3x3_small.cu, UP modes).
-#: Off by default: 4.8 ms vs 3.6 ms for concat + halo conv at 48 maps -- 32 input channels on mma.sync.
-FUSED_TAIL = __import__("os").environ.get("EDS_FUSED_TAIL", "0") != "0"
+#: least WIDE_MIN_HW on its short side and the reduction has at least WIDE_MIN_CIN channels
+WIDE_MIN_HW = 64
+WIDE_MIN_CIN = 16
 
 
 #: when set to a list, every launch appends (kernel class, CUDA event recorded right after it on the launching
@@ -308,9 +300,10 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], strid
            impl: str = "auto", x1: Optional[torch.Tensor] = None, groups: int = 1) -> torch.Tensor:
     """x [N,H,W,C], w [Cout,R,S,C] (same dtype as x) -> [N,Ho,Wo,Cout].
 
-    impl: "tc" = tcgen05 implicit GEMM (bf16 only; picks the generic, halo-reuse or dw-grouped wide-N kernel by
-    layer shape), "halo" / "wide" = force that kernel, "simt" = CUDA-core kernel,
-    "auto" = tc for bf16 activations, simt for fp32 (the fp32 parity mode).
+    impl: "tc" = bf16 kernels picked by layer shape (the mma.sync kernel of conv3x3_small.cu for the 16-channel
+    tail, else the tcgen05 generic, halo-reuse or dw-grouped wide-N implicit GEMM), "igemm" / "halo" / "wide" =
+    force that tcgen05 kernel, "simt" = CUDA-core kernel, "auto" = tc for bf16 activations, simt for fp32 (the
+    fp32 parity mode).
 
     groups > 1 (ResNeXt 3x3): always the grouped kernels, w [Cout,R,S,64] from pack_grouped_weights on the tensor
     cores, w [Cout,R,S,C/groups] on the CUDA cores.  A shape the grouped tcgen05 kernel does not take raises.
@@ -330,7 +323,7 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], strid
         out = torch.empty((N, Ho, Wo, Cout), dtype=x.dtype, device=x.device)
     if impl == "auto":
         impl = "tc" if x.dtype == torch.bfloat16 else "simt"
-    if impl in ("tc", "halo", "wide"):
+    if impl in ("tc", "igemm", "halo", "wide"):
         if x.dtype != torch.bfloat16:
             raise TypeError("the tcgen05 kernel takes bf16 activations")
         trace = CONV_TRACE
@@ -339,17 +332,17 @@ def conv2d(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], strid
             ev0.record()
         # measured (48 maps): 16 -> 16 @1024^2 1.7 ms here vs 2.4 ms on the tcgen05 halo kernel; with 32 input
         # channels the legacy mma.sync pipe (~100 TFLOP/s in these kernels) loses to tcgen05 (32 -> 32 @512^2:
-        # 2.2 ms vs 0.6 ms), so only the 16-channel layers are routed here
-        if (impl == "tc" and SMALL_CONV and Cin == 16 and x1 is None and residual is None and R == 3 and S == 3 and
-                stride == 1 and pad == 1 and _lib.load().eds_conv3x3_small_supported(Cin, Cout)):
+        # 2.2 ms vs 0.6 ms), so the small kernel takes only 16 input channels
+        if (impl == "tc" and x1 is None and residual is None and R == 3 and S == 3 and stride == 1 and pad == 1 and
+                _lib.load().eds_conv3x3_small_supported(Cin, Cout)):
             return conv3x3_small(x, w, bias, relu, out=out)
         # measured at 48 maps (scripts/dev_wide_probe.py, wide vs halo): 448 -> 64 @512^2 5.17 ms vs 6.02, 320 -> 32
         # 2.38 vs 4.31, 896 -> 64 @256^2 2.47 vs 2.92, 64 -> 64 @512^2 (weights resident) 1.33 vs 1.51, 32 -> 32 0.57
         # vs 0.67, 32 -> 16 @1024^2 1.00 vs 1.24
-        wide = impl == "wide" or (impl == "tc" and WIDE_CONV and min(H, W_) >= WIDE_MIN_HW and
+        wide = impl == "wide" or (impl == "tc" and min(H, W_) >= WIDE_MIN_HW and
                                   Cin + C1 >= WIDE_MIN_CIN and
                                   _lib.load().eds_conv3x3_wide_supported(Cin + C1, Cout, R, S, stride, pad))
-        halo = not wide and (impl == "halo" or (impl == "tc" and HALO_MIN_HW and min(H, W_) >= HALO_MIN_HW and
+        halo = not wide and (impl == "halo" or (impl == "tc" and min(H, W_) >= HALO_MIN_HW and
                                                 _lib.load().eds_conv3x3_halo_supported(Cin + C1, Cout, R, S, stride, pad)))
         _TAG[0] = "conv3x3_wide (tcgen05)" if wide else "conv3x3_halo (tcgen05)" if halo else \
             f"conv_igemm {R}x{R} (tcgen05)"
@@ -461,17 +454,13 @@ def affine_rows(m: torch.Tensor, w: torch.Tensor, b: Optional[torch.Tensor], out
 
 
 def conv3x3_small(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], relu: bool = True,
-                  up_mode: int = _lib.UP_NONE, cgate: Optional[torch.Tensor] = None,
-                  sgate: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Decoder-tail 3x3 convolution (C, Cout in {16, 32}, bf16) on mma.sync; with up_mode nearest / bilinear the
-    input is the LOW-resolution map [N,h,w,C] (optionally with its pending SCSE gate) and the x2 upsampling is
-    fused into the tile loader.  -> [N, H, W, Cout]."""
-    _chk(x, w, bias, cgate, sgate, out)
-    N, h, w_, Cin = x.shape
+                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Decoder-tail 3x3 s1 p1 convolution on mma.sync: x [N,H,W,16] bf16, w [Cout,3,3,16] with Cout in {16, 32}
+    -> [N, H, W, Cout]."""
+    _chk(x, w, bias, out)
+    N, H, W_, Cin = x.shape
     Cout = w.shape[0]
     assert x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and w.shape == (Cout, 3, 3, Cin)
-    up = 1 if up_mode == _lib.UP_NONE else 2
-    H, W_ = up * h, up * w_
     if out is None:
         out = torch.empty((N, H, W_, Cout), dtype=x.dtype, device=x.device)
     trace = CONV_TRACE
@@ -479,8 +468,8 @@ def conv3x3_small(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor]
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
     _TAG[0] = "conv3x3_small (mma.sync)"
-    check(_lib.lib().eds_conv3x3_small_bf16(_p(x), _p(cgate), _p(sgate), up_mode, N, H, W_, Cin, _p(w), _p(bias), Cout,
-                                            int(relu), _p(out), _stream()))
+    check(_lib.lib().eds_conv3x3_small_bf16(_p(x), N, H, W_, Cin, _p(w), _p(bias), Cout, int(relu), _p(out),
+                                            _stream()))
     if trace is not None:
         ev1.record()
         trace.append((2.0 * N * H * W_ * Cout * 9 * Cin, ev0, ev1, (N, H, W_, Cin, Cout, 3, 1)))

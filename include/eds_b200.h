@@ -285,16 +285,12 @@ EDS_API int eds_conv3x3_wide_bf16_2src(const void* x0, int C0, const void* x1, i
                                        const void* w, const float* bias, int Cout, int relu, const void* residual,
                                        void* y, void* stream);
 
-/* 3x3 / stride 1 / pad 1 convolution for the full-resolution decoder tail (C, Cout in {16, 32}; bf16; w
- * [Cout][3][3][C], fp32 bias, optional ReLU) on mma.sync, optionally fused with the x2 upsampling of a gated
- * low-resolution input (conv3x3_small.cu): up_mode EDS_UP_NONE -> x is [N][H][W][C]; EDS_UP_NEAREST /
- * EDS_UP_BILINEAR -> x is [N][H/2][W/2][C] and the kernel convolves up2x(x * (cgate[n][c] + sgate[n][p]))
- * without materialising it (cgate / sgate NULL = plain input).  Replaces interpolate + conv1 + conv2 of the
- * last DecoderBlock (unetplusplusstar.py:151-161).  y: [N][H][W][Cout]. */
+/* 3x3 / stride 1 / pad 1 convolution for the full-resolution decoder tail on mma.sync (conv3x3_small.cu):
+ * x [N][H][W][C], w [Cout][3][3][C] bf16, fp32 bias (may be NULL), optional ReLU -> y [N][H][W][Cout] bf16.
+ * eds_conv3x3_small_supported returns 1 for C = 16 and Cout in {16, 32}, the only shapes it takes. */
 EDS_API int eds_conv3x3_small_supported(int C, int Cout);
-EDS_API int eds_conv3x3_small_bf16(const void* x, const float* cgate, const float* sgate, int up_mode, int N, int H,
-                                   int W, int C, const void* w, const float* bias, int Cout, int relu, void* y,
-                                   void* stream);
+EDS_API int eds_conv3x3_small_bf16(const void* x, int N, int H, int W, int C, const void* w, const float* bias,
+                                   int Cout, int relu, void* y, void* stream);
 
 /* Convolution of the channel concatenation cat(x0 [N][H][W][C0], x1 [N][H][W][C1]) without building it:
  * the K loop walks the channel chunks of x0, then of x1, through two tensor maps (stride 1; w is

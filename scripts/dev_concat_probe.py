@@ -1,5 +1,4 @@
-"""Time the decoder concat (both parts, split destination) on the benchmark's layer shapes (dev tool).
-Run twice: EDS_CONCAT_SKIP_LEAN=0 / 1."""
+"""Time the decoder concat (both parts, split destination) on the benchmark's layer shapes (dev tool)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -13,7 +12,6 @@ layers = [("x_1_3", 256, 256, True, [(64, True), (64, True), (64, False)]),
           ("x_1_2", 128, 512, False, [(256, True), (256, False)]),
           ("x_0_2", 128, 128, False, [(256, True), (256, True), (256, False)]),
           ("x_2_2", 128, 512, False, [(256, False)])]
-tag = os.environ.get("EDS_CONCAT_SKIP_LEAN", "1")
 tot = 0.0
 for name, h, C0, xg, skips in layers:
     def src(n, hh, C, gated):
@@ -36,6 +34,6 @@ for name, h, C0, xg, skips in layers:
     tot += ms
     out_b = N * (2 * h) ** 2 * Ctot * 2
     in_b = N * h * h * C0 * 2 + N * (2 * h) ** 2 * sum(C for C, _ in skips) * 2
-    print(f"lean={tag} {name}: {ms:.3f} ms  ({(in_b + out_b) / ms / 1e6:.0f} GB/s read+write)", flush=True)
+    print(f"{name}: {ms:.3f} ms  ({(in_b + out_b) / ms / 1e6:.0f} GB/s read+write)", flush=True)
     del srcs, cg1, sg1
-print(f"lean={tag} total {tot:.3f} ms")
+print(f"total {tot:.3f} ms")

@@ -18,5 +18,5 @@ for (H, C, Cout, R) in [(256, 64, 256, 1), (128, 128, 512, 1), (64, 256, 1024, 1
     y = torch.empty(N, H, H, Cout, device='cuda', dtype=torch.bfloat16)
     ms = timeit(lambda: K.conv2d(x, w, b, 1, R // 2, True, None, out=y, impl='tc'))
     by = (x.numel() + y.numel()) * 2
-    print(f"stbufs={os.environ.get('EDS_IGEMM_STBUFS','2')} N{N} {H} C{C}->{Cout} k{R}: {ms:.3f} ms {by/ms/1e6:.0f} GB/s", flush=True)
+    print(f"N{N} {H} C{C}->{Cout} k{R}: {ms:.3f} ms {by/ms/1e6:.0f} GB/s", flush=True)
     del x, w, y

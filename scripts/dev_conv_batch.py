@@ -18,5 +18,5 @@ for (H, C, Cout, R) in [(512, 448, 64, 3), (512, 320, 32, 3), (512, 64, 64, 3), 
     y = torch.empty(N, H, H, Cout, device='cuda', dtype=torch.bfloat16)
     ms = timeit(lambda: K.conv2d(x, w, b, 1, R // 2, True, None, out=y, impl='tc'))
     fl = 2.0 * N * H * H * C * Cout * R * R
-    print(f"promo={os.environ.get('EDS_L2_PROMO','256')} N{N} {H} C{C}->{Cout} k{R}: {ms:.3f} ms {fl/ms/1e9:.0f} TF", flush=True)
+    print(f"N{N} {H} C{C}->{Cout} k{R}: {ms:.3f} ms {fl/ms/1e9:.0f} TF", flush=True)
     del x, w, y

@@ -1,5 +1,5 @@
-"""One 48-map pass (6 tiles x 8 D4 views, proposed net, bf16, CUDA graph) timed in isolation (dev tool for A/B runs
-with environment switches such as EDS_SE_EPILOGUE / EDS_CONCAT_SKIP_LEAN)."""
+"""One 48-map pass (6 tiles x 8 D4 views, proposed net, bf16, CUDA graph) timed in isolation (dev tool; the line it
+prints starts with the EDS_* environment it ran under)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))

@@ -16,9 +16,8 @@ def conv(N, H, W, C, Cout, R, impl, stride=1, x1c=0, res=False):
 conv(2, 20, 24, 64, 256, 3, "tc"); conv(1, 33, 17, 128, 80, 1, "tc", res=True); conv(2, 16, 16, 64, 128, 3, "tc", stride=2)
 conv(1, 24, 24, 64, 512, 3, "tc", x1c=192); conv(3, 40, 20, 64, 32, 3, "halo", res=True); conv(1, 70, 13, 128, 64, 3, "halo", x1c=64)
 conv(1, 66, 30, 16, 16, 3, "halo"); conv(2, 64, 64, 32, 16, 3, "halo")
-x = torch.randn(2, 21, 19, 32, device=dev).bfloat16()
-K.conv3x3_small(x, torch.randn(16, 3, 3, 32, device=dev).bfloat16(), torch.zeros(16, device=dev), True, _lib.UP_BILINEAR,
-                torch.rand(2, 32, device=dev), torch.rand(2, 21, 19, device=dev))
+K.conv3x3_small(torch.randn(2, 21, 19, 16, device=dev).bfloat16(), torch.randn(32, 3, 3, 16, device=dev).bfloat16(),
+                torch.zeros(32, device=dev), True)
 K.conv3x3_small(torch.randn(2, 37, 45, 16, device=dev).bfloat16(), torch.randn(16, 3, 3, 16, device=dev).bfloat16(), None, True)
 srcs = [(torch.randn(2, 7, 5, 64, device=dev).bfloat16(), torch.rand(2, 64, device=dev), torch.rand(2, 7, 5, device=dev)),
         (torch.randn(2, 14, 10, 32, device=dev).bfloat16(), None, None)]

@@ -31,6 +31,14 @@ def test_library_loads_and_exports_every_declared_symbol():
     assert lib.eds_version() >= 100
 
 
+def test_small_conv_eligibility_is_a_host_decision():
+    """eds_conv3x3_small_supported needs no GPU: the mma.sync tail kernel takes 16 input channels and 16 or 32
+    output channels; 32-channel inputs go to the tcgen05 kernels (kernels.conv2d)."""
+    lib = _lib.load()
+    assert lib.eds_conv3x3_small_supported(16, 16) and lib.eds_conv3x3_small_supported(16, 32)
+    assert not lib.eds_conv3x3_small_supported(32, 16) and not lib.eds_conv3x3_small_supported(32, 32)
+
+
 def test_compute_entries_fail_loudly_without_a_gpu():
     if torch.cuda.is_available():
         pytest.skip("GPU present")

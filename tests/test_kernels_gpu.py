@@ -142,12 +142,7 @@ def test_conv3x3_halo_bf16(case):
     tol = 1e-2 * max(1.0, ref.abs().max().item())
     assert err < tol, f"halo conv max abs err {err} (tol {tol}), rel {rel_err(y, ref)}"
     assert rel_err(y, ref) < 4e-3
-    old = K.HALO_MIN_HW, K.WIDE_CONV
-    K.HALO_MIN_HW, K.WIDE_CONV = 0, False           # impl="tc" then means the generic kernel
-    try:
-        y2 = K.conv2d(x, w, b, 1, 1, relu, res, impl="tc")
-    finally:
-        K.HALO_MIN_HW, K.WIDE_CONV = old
+    y2 = K.conv2d(x, w, b, 1, 1, relu, res, impl="igemm")
     assert (y.float() - y2.float()).abs().max().item() < tol
 
 
@@ -601,31 +596,19 @@ def test_concat_gated_split_equals_single_map(mode):
     assert torch.equal(up2, one2[..., :64].contiguous()) and torch.equal(skip2, one2[..., 64:].contiguous())
 
 
-@pytest.mark.parametrize("cin,cout", [(32, 16), (16, 16), (32, 32), (16, 32)])
-@pytest.mark.parametrize("up", [2, 0, 1])             # EDS_UP_NONE, nearest, bilinear
-@pytest.mark.parametrize("gated", [False, True])
-def test_conv3x3_small_with_fused_upsample(cin, cout, up, gated):
-    """Decoder-tail kernel == conv3x3(up2x(gated x)) in fp32 on the same bf16 data; ragged tiles (sizes that
-    are not multiples of the 16 x 32 output tile) and several images."""
-    N, h, w = 3, 21, 19
+@pytest.mark.parametrize("cout", [16, 32])
+def test_conv3x3_small(cout):
+    """Decoder-tail kernel == conv3x3(x) in fp32 on the same bf16 data; ragged tiles (sizes that are not
+    multiples of the 16 x 32 output tile) and several images."""
+    N, h, w, cin = 3, 21, 19, 16
     x = rnd(N, h, w, cin, seed=50).bfloat16()
     wt = rnd(cout, 3, 3, cin, seed=51, scale=1.0 / math.sqrt(9 * cin)).bfloat16()
     b = rnd(cout, seed=52)
-    cg = sg = None
-    val = x.float()
-    if gated:
-        cg = torch.rand(N, cin, device=DEV, generator=torch.Generator(DEV).manual_seed(53))
-        sg = torch.rand(N, h, w, device=DEV, generator=torch.Generator(DEV).manual_seed(54))
-        val = val * (cg.view(N, 1, 1, cin) + sg.unsqueeze(-1))
-    inp = nchw(val)
-    if up == 1:
-        inp = F.interpolate(inp, scale_factor=2, mode="bilinear", align_corners=False)
-    elif up == 0:
-        inp = F.interpolate(inp, scale_factor=2, mode="nearest")
+    inp = nchw(x.float())
     ref = nhwc(F.relu(F.conv2d(inp, wt.float().permute(0, 3, 1, 2), b, padding=1)))
-    y = K.conv3x3_small(x, wt, b, True, up, cg, sg)
+    y = K.conv3x3_small(x, wt, b, True)
     assert y.shape == ref.shape
-    # the kernel rounds the (gated, upsampled) input tile to bf16 before the MMA: compare against that too
+    # the kernel rounds the input tile to bf16 before the MMA: compare against that too
     ref_r = nhwc(F.relu(F.conv2d(inp.bfloat16().float(), wt.float().permute(0, 3, 1, 2), b, padding=1)))
     assert rel_err(y, ref) < 8e-3 and rel_err(y, ref_r) < 4e-3
     assert (y.float() - ref_r).abs().max().item() < 2e-2 * max(1.0, ref.abs().max().item())
@@ -636,12 +619,7 @@ def test_conv3x3_small_matches_implicit_gemm_at_tail_size():
     wt = rnd(16, 3, 3, 16, seed=56, scale=1.0 / 12).bfloat16()
     b = rnd(16, seed=57)
     y = K.conv3x3_small(x, wt, b, True)
-    old = K.SMALL_CONV
-    K.SMALL_CONV = False
-    try:
-        y2 = K.conv2d(x, wt, b, 1, 1, True, None, impl="tc")
-    finally:
-        K.SMALL_CONV = old
+    y2 = K.conv2d(x, wt, b, 1, 1, True, None, impl="wide")
     assert (y.float() - y2.float()).abs().max().item() < 2e-2
 
 
