@@ -24,9 +24,6 @@ from .. import _lib, kernels as K
 from .spec import dense_decoder_blocks
 
 IDENTITY_VIEW = [(1, 0, 0, 0, 1, 0)]
-#: on the tensor-core path, SE bottleneck maps of at least this many pixels get the block's tail (scale, residual,
-#: ReLU) in conv3's epilogue; smaller ones run conv3 and se_scale_add_relu as separate passes
-SE_EPILOGUE_MIN_PIXELS = 256 * 256
 BN_EPS = 1e-5
 
 
@@ -340,17 +337,12 @@ class Engine:
         if self.conv_impl == "tc":
             # conv3 (1x1 + folded BN) has no activation, so the channel means its SE module squeezes are an affine
             # function of the channel means of conv3's INPUT (a quarter of the channels): the gate is known before
-            # conv3 runs and the squeeze never re-reads the 4x wider map.  On the large maps scale + residual + ReLU
-            # then happen on conv3's accumulators (the pre-activation map is never written); on the small ones the
-            # epilogue's residual path costs more than the separate pass it replaces (scripts/dev_se_probe.py: 48
-            # maps, fused vs conv3 + scale: 1.39 vs 1.44 ms at 256^2, 0.76 vs 0.73 at 128^2, 0.42 vs 0.38 at 64^2)
+            # conv3 runs and the squeeze never re-reads the 4x wider map.  Scale + residual + ReLU then happen on
+            # conv3's accumulators: the pre-activation map is never written.
             w3, b3 = self.w[p + ".conv3"]
             squeeze = K.affine_rows(K.channel_mean(out), self.w[p + ".conv3.f32"][0], b3)
             gate = K.se_gate(squeeze, *self.w[p + ".se"])
-            if out.shape[1] * out.shape[2] >= SE_EPILOGUE_MIN_PIXELS:
-                return K.conv1x1_se(out, w3, b3, gate, res)
-            out = self._cv(out, p + ".conv3")
-            return K.se_scale_add_relu(out, gate, res, out=out)
+            return K.conv1x1_se(out, w3, b3, gate, res)
         out = self._cv(out, p + ".conv3")
         gate = K.se_gate(K.channel_mean(out), *self.w[p + ".se"])
         return K.se_scale_add_relu(out, gate, res, out=out)

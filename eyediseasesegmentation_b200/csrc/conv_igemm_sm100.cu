@@ -21,9 +21,12 @@
 //            input chunk n, so the K loop is the taps alone; the A box starts at channel n * 64 (a_nt_ch) and B is a
 //            block-diagonal [Cout][taps][64] matrix (zeros outside each output channel's group).
 // Persistent: grid = min(#tiles, #SMs), the TMA ring runs across tile boundaries.
-// Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
-// warps 2-9 = epilogue (TMEM -> registers -> bias/residual/ReLU -> bf16 -> swizzled shared memory ->
-// one TMA bulk tensor store per 64-channel group).
+// Warp roles (352 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer,
+// warps 2-9 = epilogue (TMEM -> registers -> bias/gate/residual/ReLU -> bf16 -> swizzled shared memory ->
+// one TMA bulk tensor store per 64-channel group), warp 10 = residual producer (TMA loads of the residual
+// tile of each group into the staging buffer its output will leave from; idle without a residual).
+// The kernel is compiled with and without the residual (kResidual), so layers without one run an epilogue with
+// no residual code: sharing one instance cost the plain 1x1 convolutions about 2 % (48 maps on a B200).
 #include "tc_ptx.cuh"
 #include <algorithm>
 #include <climits>
@@ -32,9 +35,10 @@
 
 namespace eds {
 
-constexpr int kIgemmThreads = 320;   // TMA warp, MMA warp, 8 epilogue warps
+constexpr int kIgemmThreads = 352;   // TMA warp, MMA warp, 8 epilogue warps, residual TMA warp
 constexpr int kMaxTaps = 9;
 constexpr int kMaxStages = 8;
+constexpr int kMaxStBufs = 4;        // staging buffers per epilogue half
 constexpr int kTileM = 128;
 
 struct IgemmParams {
@@ -45,15 +49,15 @@ struct IgemmParams {
     CUtensorMap b_map;
     const float* bias;
     const float* gate;      // optional [N][Cout]: y = relu((acc + bias) * gate[n][co] + residual)  (SE scale fused)
-    const __nv_bfloat16* residual;
     __nv_bfloat16* y;
     int taps, C, block_k, k_chunks, block_n, n_tiles;
     int tw_log2, th_log2, TW, TH, TN;
     int tiles_w, tiles_h;
     int N, Ho, Wo, Cout, relu;
     CUtensorMap y_map;      // output [Cout][Wo][Ho][N], box [st_ch][TW][TH][TN]
+    CUtensorMap r_map;      // residual: the dims, strides, box and swizzle of y_map
     int total_tiles;        // after y_map: nvcc 12.9 then spills 76 / 96 B (stores / loads) instead of 84 / 112 B
-    int st_ch, st_bytes, st_bufs, st_mode;   // epilogue staging: channels per TMA store, bytes per buffer, buffers per half, swizzle mode
+    int st_ch, st_bytes, st_bufs, st_bufs_log2, st_mode;   // epilogue staging: channels per TMA store, bytes per buffer, buffers per half, swizzle mode
     int stages, a_stage_bytes, b_stage_bytes, tmem_cols;
     uint32_t idesc;
     uint32_t desc_hi;  // upper 32 bits of the smem descriptor (SBO, version, swizzle mode)
@@ -69,6 +73,7 @@ __device__ __forceinline__ void mbar_arrive_cta(uint64_t* bar) {
 // the accumulator is double-buffered in TMEM (2 x block_n columns), so the epilogue of tile t
 // overlaps the main loop of tile t + 1 and the per-CTA set-up (barriers, TMEM allocation,
 // descriptor prefetch) is paid once per SM instead of once per tile.
+template <bool kResidual>
 __global__ void __launch_bounds__(kIgemmThreads, 1)
 conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -76,12 +81,13 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const int stage_bytes = p.a_stage_bytes + p.b_stage_bytes;
     uint8_t* staging = smem + (size_t)p.stages * stage_bytes;          // [2 halves][st_bufs][st_bytes]
-    uint8_t* res_stage = staging + (size_t)2 * p.st_bufs * p.st_bytes; // [2 halves][2][st_bytes] when there is a residual
-    uint64_t* full_bar = reinterpret_cast<uint64_t*>(res_stage + (p.residual ? (size_t)4 * p.st_bytes : 0));
+    uint64_t* full_bar = reinterpret_cast<uint64_t*>(staging + (size_t)2 * p.st_bufs * p.st_bytes);
     uint64_t* empty_bar = full_bar + kMaxStages;
     uint64_t* tmem_full_bar = empty_bar + kMaxStages;      // [2]
     uint64_t* tmem_empty_bar = tmem_full_bar + 2;          // [2]
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_empty_bar + 2);
+    uint64_t* res_full_bar = tmem_empty_bar + 2;           // [2 halves][kMaxStBufs]: residual tile landed
+    uint64_t* res_free_bar = res_full_bar + 2 * kMaxStBufs; // [2 halves][kMaxStBufs]: the store has read the buffer
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_free_bar + 2 * kMaxStBufs);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int num_k_iters = p.taps * p.k_chunks;
@@ -97,6 +103,10 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
         for (int b = 0; b < 2; ++b) {
             mbar_init(&tmem_full_bar[b], 1);
             mbar_init(&tmem_empty_bar[b], 8);      // one arrival per epilogue warp
+        }
+        for (int b = 0; b < 2 * kMaxStBufs; ++b) {
+            mbar_init(&res_full_bar[b], 1);
+            mbar_init(&res_free_bar[b], 1);        // the issuing thread of the half
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -176,11 +186,14 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
             if (elect_one()) umma_commit(&tmem_full_bar[buf]);
             __syncwarp();
         }
-    } else {
+    } else if (warp < 10) {
         // ===== epilogue: 8 warps; warp w may only touch TMEM lanes [32 (w % 4), +32), so two warps share
         // a lane quadrant and the two "halves" (4 warps = 128 rows each) take alternate channel groups.
         // A group of st_ch channels of the 128-pixel tile is staged in shared memory in the TMA
         // swizzle and leaves as ONE bulk tensor store (coalesced, clipped at the map edge by TMA).
+        // With a residual the staging buffer of a group already holds the group's residual tile (loaded by
+        // warp 10 in the same swizzle, zero-filled outside the map): each thread reads its row's chunks and
+        // overwrites them with the result, in place.
         const int q = warp & 3;
         const int half = (warp - 2) >> 2;
         const int m = q * 32 + lane;
@@ -193,40 +206,7 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
         const uint32_t swz = p.st_mode == 0 ? (uint32_t)(m & 7) : (p.st_mode == 1 ? (uint32_t)((m >> 1) & 3) : (uint32_t)((m >> 2) & 1));
         uint8_t* my_stage = staging + (size_t)half * p.st_bufs * p.st_bytes;
         const bool issuer = (warp - 2) % 4 == 0 && lane == 0;      // first warp of the half
-        // Residual (skip connection / SE bottleneck tail): the [128 pixels][st_ch] tile of a group is fetched
-        // COOPERATIVELY with cp.async, 16-byte chunk by chunk in row-major order of the staging layout (a warp copies
-        // whole 128-byte pixel rows: coalesced), into one of two buffers of this half, ONE GROUP AHEAD of its use.
-        // (A lane owns one PIXEL: reading its residual directly touched 32 different lines per load instruction and
-        // doubled the time of the SE bottleneck's conv3 once scale + residual + ReLU moved into this epilogue.)
-        uint8_t* my_res = res_stage + (size_t)half * 2 * p.st_bytes;
-        const int hid = (warp - 2) % 4 * 32 + lane;                // thread index inside the half (0..127)
-        auto fetch_residual = [&](int tile_, int grp_, uint8_t* dstbuf) {
-            const int cpr = row_bytes >> 4;                         // 16-byte chunks per staging row: 8 / 4 / 2
-            const int n_tile_ = tile_ % p.n_tiles;
-            int m_tile_ = tile_ / p.n_tiles;
-            const int w0_ = (m_tile_ % p.tiles_w) * p.TW;
-            m_tile_ /= p.tiles_w;
-            const int h0_ = (m_tile_ % p.tiles_h) * p.TH, n0_ = (m_tile_ / p.tiles_h) * p.TN;
-            const int64_t c0_ = (int64_t)n_tile_ * p.block_n + grp_ * p.st_ch;
-#pragma unroll 1
-            for (int qc = hid; qc < kTileM * cpr; qc += 128) {
-                const int rr = qc / cpr, jc = qc - rr * cpr;
-                const int rw = w0_ + (rr & (p.TW - 1)), rh = h0_ + ((rr >> p.tw_log2) & (p.TH - 1));
-                const int rn = n0_ + (rr >> (p.tw_log2 + p.th_log2));
-                if (rw < p.Wo && rh < p.Ho && rn < p.N) {
-                    const uint32_t sw = p.st_mode == 0 ? (uint32_t)(rr & 7)
-                                      : (p.st_mode == 1 ? (uint32_t)((rr >> 1) & 3) : (uint32_t)((rr >> 2) & 1));
-                    const __nv_bfloat16* src = p.residual + (((int64_t)rn * p.Ho + rh) * p.Wo + rw) * p.Cout + c0_ + jc * 8;
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(
-                                     dstbuf + (size_t)rr * row_bytes + (((uint32_t)jc ^ sw) << 4))), "l"(src) : "memory");
-                }
-            }
-        };
         int t = 0, sbuf = 0, gcount = 0;
-        if (p.residual) {                                           // prologue: the first group of this half
-            if ((int)blockIdx.x < p.total_tiles && half < n_groups) fetch_residual(blockIdx.x, half, my_res);
-            asm volatile("cp.async.commit_group;" ::: "memory");
-        }
         for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x, ++t) {
             const int buf = t & 1;
             const int n_tile = tile % p.n_tiles;
@@ -261,26 +241,23 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                         bv[i][e] = (p.bias && i < n16)
                                        ? __ldg(reinterpret_cast<const float4*>(p.bias + co0 + grp * p.st_ch + i * 16) + e)
                                        : make_float4(0.f, 0.f, 0.f, 0.f);
-                // the store that last read this staging buffer must have finished reading it
-                if (issuer) {
-                    if (p.st_bufs == 2) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(1) : "memory");
-                    else asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(0) : "memory");
-                }
-                asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");
-                // residual tile: the copy of THIS group was issued one group ago (or in the prologue); issue the
-                // next group's now so that it flies during this group's work
-                const uint8_t* rcur = my_res + (size_t)(gcount & 1) * p.st_bytes;
-                if (p.residual) {
-                    int ntile = tile, ngrp = grp + 2;
-                    if (ngrp >= n_groups) { ntile = tile + gridDim.x; ngrp = half; }
-                    if (ntile < p.total_tiles && ngrp < n_groups) fetch_residual(ntile, ngrp, my_res + (size_t)((gcount + 1) & 1) * p.st_bytes);
-                    asm volatile("cp.async.commit_group;" ::: "memory");          // (possibly empty) keeps the count uniform
+                if (kResidual) {
+                    // the store of the previous group has read its buffer: warp 10 may refill it
+                    if (issuer && gcount > 0) {
+                        asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(0) : "memory");
+                        mbar_arrive_cta(&res_free_bar[half * kMaxStBufs + ((sbuf - 1) & (p.st_bufs - 1))]);
+                    }
+                    // this group's residual tile has landed in its staging buffer (use gcount / st_bufs of it)
+                    mbar_wait(&res_full_bar[half * kMaxStBufs + sbuf], (uint32_t)((gcount >> p.st_bufs_log2) & 1));
+                } else {
+                    // the store that last read this staging buffer must have finished reading it
+                    if (issuer) {
+                        if (p.st_bufs == 2) asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(1) : "memory");
+                        else asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(0) : "memory");
+                    }
+                    asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");
                 }
                 tmem_ld_wait();
-                if (p.residual) {
-                    asm volatile("cp.async.wait_group 1;" ::: "memory");           // everything but the prefetch just issued
-                    asm volatile("bar.sync %0, 128;" ::"r"(1 + half) : "memory");  // ... of every thread of the half
-                }
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
                     if (i >= n16) break;
@@ -302,12 +279,12 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                             v[4 * e] *= gg.x; v[4 * e + 1] *= gg.y; v[4 * e + 2] *= gg.z; v[4 * e + 3] *= gg.w;
                         }
                     }
-                    if (p.residual) {                          // this lane's own row of the parked residual tile
-                        const uint32_t jr = (uint32_t)c16 >> 3;
-                        const uint8_t* rrow = rcur + (size_t)m * row_bytes;
+                    const uint32_t j = (uint32_t)c16 >> 3;          // 16-byte chunk index of the first 8 channels
+                    uint8_t* rowp = sdst + (size_t)m * row_bytes;
+                    if (kResidual) {                          // this thread's row of the residual tile
                         float r0[8], r1[8];
-                        Vec8<__nv_bfloat16>::ld(reinterpret_cast<const __nv_bfloat16*>(rrow + ((jr ^ swz) << 4)), r0);
-                        Vec8<__nv_bfloat16>::ld(reinterpret_cast<const __nv_bfloat16*>(rrow + (((jr + 1) ^ swz) << 4)), r1);
+                        Vec8<__nv_bfloat16>::ld(reinterpret_cast<const __nv_bfloat16*>(rowp + ((j ^ swz) << 4)), r0);
+                        Vec8<__nv_bfloat16>::ld(reinterpret_cast<const __nv_bfloat16*>(rowp + (((j + 1) ^ swz) << 4)), r1);
 #pragma unroll
                         for (int e = 0; e < 8; ++e) { v[e] += r0[e]; v[8 + e] += r1[e]; }
                     }
@@ -325,8 +302,6 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
                             h1p[e] = __floats2bfloat162_rn(v[8 + 2 * e], v[8 + 2 * e + 1]);
                         }
                     }
-                    const uint32_t j = (uint32_t)c16 >> 3;          // 16-byte chunk index of the first 8 channels
-                    uint8_t* rowp = sdst + (size_t)m * row_bytes;
                     *reinterpret_cast<uint4*>(rowp + ((j ^ swz) << 4)) = o0;
                     *reinterpret_cast<uint4*>(rowp + (((j + 1) ^ swz) << 4)) = o1;
                 }
@@ -348,6 +323,32 @@ conv_igemm_kernel(const __grid_constant__ IgemmParams p) {
             if (lane == 0) mbar_arrive_cta(&tmem_empty_bar[buf]);
         }
         if (issuer) asm volatile("cp.async.bulk.wait_group %0;" ::"n"(0) : "memory");    // stores complete before exit
+    } else if (kResidual && lane == 0) {
+        // ===== residual producer: walks the tiles and groups in the epilogue's order and loads the residual tile
+        // of group g of half h into staging buffer g % st_bufs of h once the store that last read that buffer has
+        // read it.  A separate warp, so that the A/B producer never waits on epilogue progress.  The half frees a
+        // buffer when it starts the group after, so with st_bufs >= 2 every wait here is for a group whose tile
+        // was loaded already: no cycle.
+        prefetch_tmap(&p.r_map);
+        const int n_groups = p.block_n / p.st_ch;
+        int gc[2] = {0, 0};
+        for (int tile = blockIdx.x; tile < p.total_tiles; tile += gridDim.x) {
+            const int n_tile = tile % p.n_tiles;
+            int m_tile = tile / p.n_tiles;
+            const int w0 = (m_tile % p.tiles_w) * p.TW;
+            m_tile /= p.tiles_w;
+            const int h0 = (m_tile % p.tiles_h) * p.TH, n0 = (m_tile / p.tiles_h) * p.TN;
+            for (int grp = 0; grp < n_groups; ++grp) {
+                const int h = grp & 1;
+                const int s = gc[h] & (p.st_bufs - 1);
+                const int use = gc[h] >> p.st_bufs_log2;
+                if (use > 0) mbar_wait(&res_free_bar[h * kMaxStBufs + s], (uint32_t)((use - 1) & 1));
+                mbar_arrive_expect_tx(&res_full_bar[h * kMaxStBufs + s], (uint32_t)p.st_bytes);
+                tma_load_4d(staging + (size_t)(h * p.st_bufs + s) * p.st_bytes, &p.r_map,
+                            &res_full_bar[h * kMaxStBufs + s], n_tile * p.block_n + grp * p.st_ch, w0, h0, n0);
+                ++gc[h];
+            }
+        }
     }
 
     tc_fence_before();
@@ -384,7 +385,9 @@ int igemm_init() {
     std::call_once(g_igemm_once, igemm_init_once);
     if (g_igemm_init_rc) return g_igemm_init_rc;
     return g_igemm_attr_once.run([](int dev) {
-        cudaError_t e = cudaFuncSetAttribute(conv_igemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(conv_igemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(conv_igemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) {
             set_error("conv_igemm: cannot opt in to 227 KB shared memory: %s", cudaGetErrorString(e));
             return (int)EDS_ERR_CUDA;
@@ -447,7 +450,6 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     p.bias = bias;
     p.gate = gate;
     EDS_REQUIRE((((uintptr_t)gate) & 15) == 0, "conv2d_igemm: gate must be 16-byte aligned");
-    p.residual = (const __nv_bfloat16*)residual;
     p.y = (__nv_bfloat16*)y;
     p.taps = R * S;
     p.C = C;
@@ -501,24 +503,30 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
     p.st_ch = (p.block_n % 64 == 0) ? 64 : (p.block_n % 32 == 0 ? 32 : 16);
     p.st_mode = p.st_ch == 64 ? 0 : (p.st_ch == 32 ? 1 : 2);
     p.st_bytes = kTileM * p.st_ch * 2;                                 // 16 / 8 / 4 KB
-    // short reductions are store-bound: overlap the bulk stores with the next groups (st_bufs per half in flight)
-    p.st_bufs = k_iters <= 8 ? 2 : 1;
-    // one persistent CTA per SM: the rest of the shared memory is one TMA ring
-    const int res_bytes = residual ? 4 * p.st_bytes : 0;               // two residual buffers per epilogue half
+    // short reductions are store-bound: overlap the bulk stores with the next groups (st_bufs per half in flight).
+    // With a residual every staging buffer also receives a residual tile ahead of its group: a half computes in
+    // one buffer, the previous group's store reads another, and the other st_bufs - 2 are filling.  The half frees
+    // a buffer only when it starts the next group, so a residual needs at least 2.
+    // Budget of the SE bottleneck tails (1x1, C = 64 / 128 / 256, Cout = 256 / 512 / 1024): block_k 64,
+    // block_n 256 -> a 16 + 32 = 48 KB A+B stage, st_ch 64 -> 16 KB staging buffers.  227 KB - 1 KB align slack
+    // - 0.5 KB barriers = 225.5 KB = 2 stages (96 KB) + 2 halves x 4 buffers (128 KB) + 1.5 KB to spare.
+    const int min_bufs = residual ? 2 : 1;
+    p.st_bufs = residual ? (k_iters <= 8 ? 4 : 2) : (k_iters <= 8 ? 2 : 1);
     // one persistent CTA per SM: the rest of the shared memory is one TMA ring of at least two stages (fewer staging
     // buffers if that is what it takes)
     int ring_budget = 0;
     for (;; p.st_bufs >>= 1) {
-        ring_budget = 227 * 1024 - 1024 /*align slack*/ - 512 /*barriers*/ - 2 * p.st_bufs * p.st_bytes - res_bytes;
-        if (ring_budget >= 2 * stage_bytes || p.st_bufs == 1) break;
+        ring_budget = 227 * 1024 - 1024 /*align slack*/ - 512 /*barriers*/ - 2 * p.st_bufs * p.st_bytes;
+        if (ring_budget >= 2 * stage_bytes || p.st_bufs == min_bufs) break;
     }
     EDS_REQUIRE(ring_budget >= 2 * stage_bytes, "conv2d_igemm: shared memory budget exhausted (stage %d B)", stage_bytes);
+    p.st_bufs_log2 = ilog2(p.st_bufs);
     p.stages = std::min(kMaxStages, ring_budget / stage_bytes);
     p.tmem_cols = std::max(32, pow2_ceil(2 * p.block_n));
     p.total_tiles = (int)n_ctas;
-    const size_t smem = (size_t)p.stages * stage_bytes + (size_t)2 * p.st_bufs * p.st_bytes + (size_t)res_bytes +
+    const size_t smem = (size_t)p.stages * stage_bytes + (size_t)2 * p.st_bufs * p.st_bytes +
                         1024 /*align slack*/ +
-                        (2 * kMaxStages + 4) * 8 + 16;
+                        (2 * kMaxStages + 4 + 4 * kMaxStBufs) * 8 + 16;
 
     // input tensor maps: one per (row parity, col parity) plane that a tap touches
     bool plane_used[4] = {false, false, false, false};
@@ -572,8 +580,12 @@ static int igemm_launch(const void* x, int C0, const void* x1, int C1, int N, in
         cuuint64_t strides[3] = {(cuuint64_t)Cout * 2, (cuuint64_t)Wo * Cout * 2, (cuuint64_t)Ho * Wo * Cout * 2};
         cuuint32_t box[4] = {(cuuint32_t)p.st_ch, (cuuint32_t)p.TW, (cuuint32_t)p.TH, (cuuint32_t)p.TN};
         if (int rc = tmap_encode_bf16(&p.y_map, y, 4, dims, strides, box, yswz, "output")) return rc;
+        if (residual) {
+            if (int rc = tmap_encode_bf16(&p.r_map, residual, 4, dims, strides, box, yswz, "residual")) return rc;
+        }
     }
-    conv_igemm_kernel<<<grid, kIgemmThreads, smem, as_stream(stream)>>>(p);
+    if (residual) conv_igemm_kernel<true><<<grid, kIgemmThreads, smem, as_stream(stream)>>>(p);
+    else conv_igemm_kernel<false><<<grid, kIgemmThreads, smem, as_stream(stream)>>>(p);
     return check_launch("conv_igemm_kernel");
 }
 
