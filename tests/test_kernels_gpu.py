@@ -12,6 +12,7 @@ import torch.nn.functional as F
 pytestmark = pytest.mark.gpu
 
 from eyediseasesegmentation_b200 import _lib, kernels as K  # noqa: E402
+from test_attention_exact_gpu import RANDOM_SHAPES, case_ref, error_bound, map_to_seq, mma_accepts, random_case  # noqa: E402,E501
 
 DEV = "cuda"
 
@@ -288,63 +289,28 @@ def test_head_conv(dtype):
 
 
 # -------------------------------------------------------------------- attention
-def attention_ref(q, k, v, rel, sim_scale, out_scale, out_shift, dqk, dv):
-    """q,k [b,h,dqk,L]; v [b,h,dv,L] -- the einsums of axial_attention_v2.py:178-213 with the
-    BatchNorms already reduced to their eval-mode scale/shift."""
-    L = q.shape[-1]
-    idx = (torch.arange(L).view(L, 1) - torch.arange(L).view(1, L) + L - 1).to(q.device)
-    emb = rel[:, idx]  # [c, x, y]
-    rq, rk, rv = emb[:dqk], emb[dqk:2 * dqk], emb[2 * dqk:]
-    qr = torch.einsum("bhid,idj->bhdj", q, rq)
-    kr = torch.einsum("bhid,idj->bhdj", k, rk)
-    dots = torch.einsum("bhid,bhij->bhdj", q, k)
-    s = sim_scale.view(1, -1, 3, 1, 1)
-    sim = qr * s[:, :, 0] + kr * s[:, :, 1] + dots * s[:, :, 2]
-    attn = torch.softmax(sim, dim=-1)
-    out = torch.einsum("bhdj,bhij->bhid", attn, v)
-    kv = torch.einsum("bhdj,idj->bhid", attn, rv)
-    b, h = q.shape[:2]
-    CO = h * dv
-    kv = kv.reshape(b, CO, L) * out_scale[:CO].view(1, -1, 1) + out_shift[:CO].view(1, -1, 1)
-    out = out.reshape(b, CO, L) * out_scale[CO:].view(1, -1, 1) + out_shift[CO:].view(1, -1, 1)
-    return kv + out  # [b, h*dv, L]
-
-
 @pytest.mark.parametrize("axis", [0, 1])
 @pytest.mark.parametrize("cross", [False, True])
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
-@pytest.mark.parametrize("shape", [(2, 16, 16, 4, 16), (1, 64, 64, 8, 64), (2, 32, 32, 4, 16), (1, 19, 19, 8, 64),
-                                   (1, 38, 38, 4, 8), (1, 24, 40, 4, 16), (1, 8, 8, 8, 64), (1, 16, 16, 2, 16)])
+@pytest.mark.parametrize("shape", RANDOM_SHAPES)
 def test_axial_attention(axis, cross, dtype, shape):
     """bf16 runs the tensor-core kernel (attention_mma.cu) where the shape allows (heads % 4 == 0, L <= 64,
     incl. lengths that are not multiples of 16 -- base_dim 19 of the vessel configs), fp32 and the
-    2-head case the CUDA-core kernel."""
-    N, H, W, heads, dv = shape
-    dqk = 8
-    L = H if axis == 0 else W
-    G = 2 * dqk + (0 if cross else dv)
-    qk = rnd(N, H, W, heads * G, seed=40, scale=0.5).to(dtype)
-    vt = rnd(N, H, W, heads * dv, seed=41, scale=0.5).to(dtype) if cross else None
-    rel = rnd(2 * dqk + dv, 2 * L - 1, seed=42, scale=0.5)
-    sim_scale = rnd(heads, 3, seed=43, scale=0.3)
-    out_scale, out_shift = rnd(2, heads * dv, seed=44), rnd(2, heads * dv, seed=45)
-    y = K.axial_attention(qk, vt, axis, heads, dqk, dv, rel, sim_scale, out_scale, out_shift)
-
-    # sequences: axis 0 -> (n, w) along h ; axis 1 -> (n, h) along w
-    def seqs(t):  # [N,H,W,Cc] -> [b, Cc, L]
-        t = t.float()
-        return t.permute(0, 2, 3, 1).reshape(N * W, -1, H) if axis == 0 else t.permute(0, 1, 3, 2).reshape(N * H, -1, W)
-
-    qk_s = seqs(qk).reshape(-1, heads, G, L)
-    q, k = qk_s[:, :, :dqk], qk_s[:, :, dqk:2 * dqk]
-    v = seqs(vt).reshape(-1, heads, dv, L) if cross else qk_s[:, :, 2 * dqk:]
-    ref = attention_ref(q, k, v, rel, sim_scale, out_scale.reshape(-1), out_shift.reshape(-1), dqk, dv)
-    if axis == 0:
-        ref = ref.reshape(N, W, heads * dv, H).permute(0, 3, 1, 2)
-    else:
-        ref = ref.reshape(N, H, heads * dv, W).permute(0, 1, 3, 2)
-    tol = 2e-4 if dtype == torch.float32 else 5e-2
-    assert (y.float() - ref).abs().max().item() < tol
+    2-head case the CUDA-core kernel.  With ReLU off and on, checked per element against the float64 reference
+    within the bound derived in test_attention_exact_gpu.error_bound (the roundings of the probabilities and of
+    the store)."""
+    c, case, qk, vt = random_case(shape, axis, cross, dtype)
+    S, heads, L, dqk = case.q.shape
+    tensor_core = dtype == torch.bfloat16 and mma_accepts(heads, dqk, c.dv, L)
+    for relu in (False, True):
+        y = K.axial_attention(qk.to(DEV), None if vt is None else vt.to(DEV), axis, heads, dqk, c.dv,
+                              case.rel.to(DEV), case.sim_scale.to(DEV), case.out_scale.to(DEV),
+                              case.out_shift.to(DEV), relu)
+        ref, _, arv, av, _ = case_ref(case, relu=relu, parts=True)
+        bound = error_bound(case, ref, arv, av, dtype, tensor_core)
+        err = (map_to_seq(y, axis).double().cpu() - ref).abs()
+        worst = float((err / bound).max())
+        assert worst <= 1, f"relu={relu}: error {worst:.2f} x the bound; max |y - ref| = {float(err.max()):.3g}"
 
 
 # ----------------------------------------------------------- TTA / paste / tile
